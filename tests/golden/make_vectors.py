@@ -16,6 +16,17 @@ tests/golden/<scene>/vectors.npz:
   adaptive_*                adaptive octree levels (min < max <= grid): triangle count, sha256 of the sorted soup
                             of getSurface, and of getSurface + retopologize
 The CPU port (oracle/) and the CUDA path are both tested against these.
+
+It also records tests/golden/<scene>/pins.npz and tests/golden/lookup_table.npz (see PIN_SCENES below):
+
+  seed5_sdf_sha             the SDF on 20000 points drawn with seed 5
+  walk5_*                   uniform walk at grid level 5 in the walk's own order: count, sha256, and after 3 descent steps
+  lattice_points            three lattice points of the 33^3 lattice
+  special_sdf / _normals    SDF and 6-tap normals on the 20^3 grid of special coordinates
+  adaptive_walk_*           the adaptive walk in its own order
+  table                     (lookup_table.npz) the 256x16 triangle table read from the reference's lookupTable.txt
+
+    python tests/golden/make_vectors.py --pins-from-port   # the same files from the port, where no reference build exists
 """
 import hashlib
 import os
@@ -64,9 +75,65 @@ def logo_vectors():
     print("logo L", L, "tris", len(soup), "adaptive", len(adaptive), "box", box)
 
 
+# tests/golden/<scene>/pins.npz: what tests/test_oracle_pinning.py's direct comparisons with the reference build compare, so
+# that they also run without one.  Recorded from the reference build, or with --pins-from-port from the port, which those
+# direct comparisons found bit-identical to it on these inputs; the file's `source` says which.
+PIN_SCENES = {"design1": (3, 5, 6), "design2": (4, 6, 6), "stress": (3, 6, 6)}      # adaptive levels: min, max, grid
+PIN_DIRECT = ("design1", "design2")
+PIN_LATTICE_POINTS = ((0, 0, 0), (32, 7, 19), (13, 32, 1))
+SPECIAL_VALUES = [0.0, -0.0, 5.0, -5.0, 1e-30, -1e-30, 1e-45, 2.0 ** -61, 2.0 ** -59, 1e37, -1e37, 3e38, np.inf, -np.inf, np.nan,
+                  1.5, -0.75, 4.9999995, 5.0000005, 1e-18]
+
+
+def special_points():
+    """The 20^3 grid of special coordinates (signed zeros, denormal / tiny / huge / infinite / NaN, centres and planes)."""
+    vals = np.array(SPECIAL_VALUES, dtype=np.float32)
+    return np.ascontiguousarray(np.stack(np.meshgrid(vals, vals, vals, indexing="ij"), axis=-1).reshape(-1, 3))
+
+
+def seed5_points():
+    return np.random.default_rng(5).uniform(-5, 5, (20000, 3)).astype(np.float32)
+
+
+def pins(orc, name):
+    box = orc.bbox(10.0)
+    out = {}
+    if name in PIN_DIRECT:
+        soup = orc.get_surface(box, 5, 5, 5)                 # walk order, unsorted
+        with np.errstate(all="ignore"):
+            sp = special_points()
+            out.update(seed5_sdf_sha=sha(orc.eval_sdf(seed5_points())), walk5_tris=len(soup), walk5_sha=sha(soup),
+                       walk5_gd3_sha=sha(orc.gradient_descent(soup, 3)),
+                       lattice_points=np.array([orc.lattice_point(box, 32, *p) for p in PIN_LATTICE_POINTS]),
+                       special_sdf=orc.eval_sdf(sp), special_normals=orc.eval_normal(sp))
+    lo, hi, grid = PIN_SCENES[name]
+    adaptive = orc.get_surface(box, lo, hi, grid)
+    out.update(adaptive_levels=np.array([lo, hi, grid]), adaptive_walk_tris=len(adaptive), adaptive_walk_sha=sha(adaptive))
+    return out
+
+
+def record_pins(flavour):
+    from oracle import build as obuild
+    from oracle.oracle import tri_table
+    for name in PIN_SCENES:
+        orc = Oracle.for_scene(scenes.materialize(name), flavour)
+        assert orc.flavour == flavour
+        np.savez_compressed(os.path.join(HERE, name, "pins.npz"), source=flavour, **pins(orc, name))
+        print(name, "pins from the", flavour)
+    if flavour == "reference":
+        table, n = orc.load_lookup_file(os.path.join(obuild.REFERENCE, "lookupTable.txt"))   # the reference's own reader
+        assert n == 820
+    else:
+        table = tri_table()
+    np.savez_compressed(os.path.join(HERE, "lookup_table.npz"), source=flavour, table=table)
+
+
 def main():
     if "--logo" in sys.argv:
         return logo_vectors()
+    if "--pins-from-port" in sys.argv:
+        return record_pins("port")
+    record_pins("reference")
     for name in scenes.names():
         scene = scenes.materialize(name)
         ref = Oracle.for_scene(scene, "reference")

@@ -1,6 +1,7 @@
 """Pins the CPU oracle (oracle/, our restatement) to the reference:
  * against the committed vectors recorded from the reference's own code (tests/golden/*/vectors.npz);
- * where a build of the reference's sources exists (oracle/_ref, this container or prebuilt), directly."""
+ * against tests/golden/*/pins.npz and tests/golden/lookup_table.npz, what the direct comparisons below compare;
+ * where a build of the reference's sources exists (oracle/_ref), directly as well."""
 import hashlib
 import os
 import re
@@ -10,6 +11,7 @@ import pytest
 
 from oracle import build as obuild
 from oracle.oracle import Oracle, tri_table
+from tests.golden import make_vectors as mv
 from tests.golden import scenes
 
 HERE = os.path.dirname(os.path.abspath(__file__))
@@ -60,16 +62,43 @@ def _ref_or_skip(name):
     return Oracle.for_scene(scenes.materialize(name), "reference")
 
 
+def _ref_or_none(name):
+    """The reference build for a direct comparison, where one exists; the stored pins are compared either way."""
+    if not obuild.have_reference() and not os.path.exists(obuild.ref_lib_path(name)):
+        return None
+    return Oracle.for_scene(scenes.materialize(name), "reference")
+
+
+def _pins(name):
+    """tests/golden/<name>/pins.npz (make_vectors.py): what the comparisons below compare with the reference build."""
+    return np.load(os.path.join(HERE, "golden", name, "pins.npz"))
+
+
+def _same_bits(a, b):
+    """Bit for bit (the sign of a zero included) wherever the values are numbers; NaN at the same places."""
+    a, b = np.asarray(a, dtype=np.float32), np.asarray(b, dtype=np.float32)
+    return np.array_equal(np.isnan(a), np.isnan(b)) and np.array_equal(a.view(np.uint32)[~np.isnan(a)], b.view(np.uint32)[~np.isnan(b)])
+
+
 @pytest.mark.parametrize("name", ["design1", "design2"])
 def test_port_equals_reference_build_directly(name):
-    ref, orc = _ref_or_skip(name), Oracle.for_scene(scenes.materialize(name), "port")
-    pts = np.random.default_rng(5).uniform(-5, 5, (20000, 3)).astype(np.float32)
+    orc, pin = Oracle.for_scene(scenes.materialize(name), "port"), _pins(name)
+    pts = mv.seed5_points()
+    box = orc.bbox(10.0)
+    a = orc.get_surface(box, 5, 5, 5)
+    assert sha(orc.eval_sdf(pts)) == str(pin["seed5_sdf_sha"])
+    assert len(a) == int(pin["walk5_tris"]) and sha(a) == str(pin["walk5_sha"])        # same triangles in the same (walk) order
+    assert sha(orc.gradient_descent(a, 3)) == str(pin["walk5_gd3_sha"])
+    assert np.array_equal([orc.lattice_point(box, 32, *p) for p in mv.PIN_LATTICE_POINTS], pin["lattice_points"])
+    ref = _ref_or_none(name)
+    if ref is None:
+        return
     assert np.array_equal(orc.eval_sdf(pts), ref.eval_sdf(pts))
     box = ref.bbox(10.0)
     a, b = orc.get_surface(box, 5, 5, 5), ref.get_surface(box, 5, 5, 5)
-    assert np.array_equal(a, b)                                   # same triangles in the same (walk) order
+    assert np.array_equal(a, b)
     assert np.array_equal(orc.gradient_descent(a, 3), ref.gradient_descent(b, 3), equal_nan=True)
-    for ix, iy, iz in ((0, 0, 0), (32, 7, 19), (13, 32, 1)):
+    for ix, iy, iz in mv.PIN_LATTICE_POINTS:
         assert np.array_equal(orc.lattice_point(box, 32, ix, iy, iz), ref.lattice_point(box, 32, ix, iy, iz))
 
 
@@ -79,19 +108,22 @@ def test_port_equals_reference_build_on_special_points(name):
     which the GPU's checked fast copy must fall back to its exact copy (tests/test_gpu_parity.py compares the GPU with the
     port there).  This closes the chain on the CPU: on the same points the port returns the bits of the reference's own
     k2.cl -- values and 6-tap normals."""
-    ref, orc = _ref_or_skip(name), Oracle.for_scene(scenes.materialize(name), "port")
-    vals = np.array([0.0, -0.0, 5.0, -5.0, 1e-30, -1e-30, 1e-45, 2.0 ** -61, 2.0 ** -59, 1e37, -1e37, 3e38, np.inf, -np.inf,
-                     np.nan, 1.5, -0.75, 4.9999995, 5.0000005, 1e-18], dtype=np.float32)
-    pts = np.ascontiguousarray(np.stack(np.meshgrid(vals, vals, vals, indexing="ij"), axis=-1).reshape(-1, 3))
+    orc, pin = Oracle.for_scene(scenes.materialize(name), "port"), _pins(name)
+    pts = mv.special_points()
     with np.errstate(all="ignore"):
-        a, b = orc.eval_sdf(pts), ref.eval_sdf(pts)
-        assert np.array_equal(a.view(np.uint32)[~np.isnan(a)], b.view(np.uint32)[~np.isnan(b)]) and np.array_equal(np.isnan(a), np.isnan(b))
-        assert np.array_equal(orc.eval_normal(pts), ref.eval_normal(pts), equal_nan=True)
+        a, n = orc.eval_sdf(pts), orc.eval_normal(pts)
+        assert _same_bits(a, pin["special_sdf"])
+        assert _same_bits(n, pin["special_normals"])
+        ref = _ref_or_none(name)
+        if ref is not None:
+            assert _same_bits(a, ref.eval_sdf(pts))
+            assert np.array_equal(n, ref.eval_normal(pts), equal_nan=True)
 
 
 def test_lookup_table_forms_agree():
     """golden loops --(oracle triangulation)--> table == the product's generated mc_table.inc
-    == (where available) the reference's own reader on its own lookupTable.txt."""
+    == the table the reference's own reader parses from its own lookupTable.txt (stored in tests/golden/lookup_table.npz;
+    read again where the reference is present)."""
     table = tri_table()
     assert (table >= 0).sum() == 820 * 3 and table[0, 0] == -1 and table[255, 0] == -1
     text = open(os.path.join(REPO, "designcsg_b200", "csrc", "mc_table.inc")).read()
@@ -99,9 +131,11 @@ def test_lookup_table_forms_agree():
     assert np.array_equal(np.array([int(v) for v in re.findall(r"-?\d+", body)]).reshape(256, 16), table)
     counts = text.split("kDcsgTriCount[256] = {")[1].split("};")[0]
     assert np.array_equal(np.array([int(v) for v in re.findall(r"\d+", counts)]), (table >= 0).sum(axis=1) // 3)
-    if os.path.exists("/root/reference/master/lookupTable.txt"):
+    assert np.array_equal(np.load(os.path.join(HERE, "golden", "lookup_table.npz"))["table"], table)
+    lookup = os.path.join(obuild.REFERENCE, "lookupTable.txt")
+    if os.path.exists(lookup):
         ref = _ref_or_skip("design1")
-        parsed, n = ref.load_lookup_file("/root/reference/master/lookupTable.txt")
+        parsed, n = ref.load_lookup_file(lookup)
         assert n == 820 and np.array_equal(parsed, table)
 
 
@@ -127,12 +161,21 @@ def _reference_retopologize(name, box, lo, hi, grid):
 @pytest.mark.parametrize("name,lo,hi,grid", [("design1", 3, 5, 6), ("design2", 4, 6, 6), ("stress", 3, 6, 6)])
 def test_adaptive_walk_and_retopologize_equal_reference_build(name, lo, hi, grid):
     """Adaptive octree levels (edge ambiguity + complex edges) and cms::retopologize: the port against the
-    reference's own sources, same triangles in the same order."""
-    ref, orc = _ref_or_skip(name), Oracle.for_scene(scenes.materialize(name), "port")
+    reference's own sources, same triangles in the same order (the walk: against the stored pins, and directly where a
+    reference build exists; retopologize, the reference's undefined behaviour, only directly)."""
+    orc, pin = Oracle.for_scene(scenes.materialize(name), "port"), _pins(name)
+    assert [int(v) for v in pin["adaptive_levels"]] == [lo, hi, grid]
+    box = orc.bbox(10.0)
+    walk = orc.get_surface(box, lo, hi, grid)
+    assert len(walk) == int(pin["adaptive_walk_tris"]) and sha(walk) == str(pin["adaptive_walk_sha"])
+    a = orc.get_surface(box, lo, hi, grid, retopologize=True)
+    assert len(a) == len(walk) * (3 * (1 << (grid - lo)) - 2)
+    ref = _ref_or_none(name)
+    if ref is None:
+        return
     box = ref.bbox(10.0)
     assert np.array_equal(orc.get_surface(box, lo, hi, grid), ref.get_surface(box, lo, hi, grid))
-    a, b = orc.get_surface(box, lo, hi, grid, retopologize=True), _reference_retopologize(name, box, lo, hi, grid)
-    assert len(a) == len(orc.get_surface(box, lo, hi, grid)) * (3 * (1 << (grid - lo)) - 2)
+    b = _reference_retopologize(name, box, lo, hi, grid)
     if b is None:
         pytest.xfail("reference retopologize (undefined behaviour) crashed in this run")
     if not np.array_equal(a, b):
