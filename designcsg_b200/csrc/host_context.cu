@@ -170,6 +170,13 @@ reload:
         }
     }
     {
+        // the projection's persistent grid is sized to the blocks that can be resident at once (registers per thread differ
+        // between the tap forms and scenes)
+        int resident = 0;
+        CUDA_TRY(ctx, cudaOccupancyMaxActiveBlocksPerMultiprocessor(&resident, (const void*)ctx->k_project, 256, (size_t)ctx->scene.private_words * 256 * 4));
+        ctx->project_blocks_per_sm = std::max(1, std::min(8, resident));
+    }
+    {
         size_t sz = 0;
         void* ptr = nullptr;
         ctx->d_camera_axes[0] = ctx->d_camera_axes[1] = ctx->d_camera_axes[2] = nullptr;

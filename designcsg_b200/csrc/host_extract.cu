@@ -529,9 +529,9 @@ int launch_project(dcsg_ctx* ctx, float* d_vertices, unsigned long long count, i
     unsigned long long* list = ctx->project_list.as<unsigned long long>() + list_offset;
     CUDA_TRY(ctx, cudaMemsetAsync(cursor, 0, 4 * sizeof(unsigned long long), stream));
     CUDA_TRY(ctx, cudaMemsetAsync(list, 0, (size_t)count * 8, stream));
-    // persistent warps: no more blocks than can be resident (8 x 256 threads per SM at most; blocks that start after the
-    // queue has drained leave at once), no more than there are batches of work
-    const unsigned long long blocks = std::min<unsigned long long>((count + 255) / 256, (unsigned long long)smCount * 8);
+    // persistent warps: no more blocks than can be resident (dcsg_build asks the occupancy calculator), no more than there
+    // are batches of work
+    const unsigned long long blocks = std::min<unsigned long long>((count + 255) / 256, (unsigned long long)smCount * ctx->project_blocks_per_sm);
     // cycle detection needs the update to be a pure function of the position: not with designs that keep mutable
     // program-scope state between evaluations; DCSG_PROJECT_ALL_STEPS=1 switches it off (measurement)
     static const bool allSteps = [] { const char* e = getenv("DCSG_PROJECT_ALL_STEPS"); return e && atoi(e) != 0; }();

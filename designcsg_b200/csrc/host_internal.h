@@ -8,6 +8,7 @@
 #include <set>
 
 #include <algorithm>
+#include <array>
 #include <chrono>
 #include <climits>
 #include <cmath>
@@ -20,6 +21,7 @@
 #include <cstring>
 #include <deque>
 #include <functional>
+#include <map>
 #include <memory>
 #include <mutex>
 #include <string>
@@ -138,9 +140,18 @@ struct Scene {
 // host_scene.cu
 bool load_scene(const std::string& dir, Scene& sc, std::string& err);
 bool scene_wants_fast_path(const Scene& sc);
-std::string assemble_source(const Scene& sc, bool fastPath, std::string& err, bool flagInShared = false);
+// tapAxes: the fast copy's normals through the per-axis forms (generate_primary_sdf_axis) instead of the rolled tap loop
+std::string assemble_source(const Scene& sc, bool fastPath, std::string& err, bool flagInShared = false, bool tapAxes = false);
 bool compile_scene(const Scene& sc, std::vector<char>& cubin, std::string& log, std::string& err, bool exactOnly = false);
 bool compile_source(const std::string& src, std::vector<char>& cubin, std::string& log);
+// what a kernel of an sm_100a cubin occupies: registers per thread, local memory (the largest stack frame of the kernel and of the
+// functions compiled into its text section), bytes of code.  Read from the ELF, no device needed.
+struct KernelFootprint {
+    int registers = -1;
+    uint32_t frameBytes = 0;
+    uint64_t textBytes = 0;
+};
+bool kernel_footprint(const std::vector<char>& cubin, const char* kernel, KernelFootprint& fp);
 void copy_log(const std::string& log, char* out, size_t cap);
 
 }  // namespace dcsg_host
@@ -156,6 +167,7 @@ struct dcsg_ctx {
     std::mutex lock;
 
     int sm_count = 0;               // multiprocessors of `device` (persistent grids are sized from it)
+    int project_blocks_per_sm = 8;  // resident blocks of dcsg_k_project per multiprocessor (dcsg_build asks the occupancy calculator)
     int node_ranks = 1;             // ranks sharing this host (set by dcsg_comm_create): they share its cores and memory bandwidth
     dcsg_progress_fn progress = nullptr;    // optional, see dcsg_set_progress_callback
     void* progress_user = nullptr;

@@ -5,6 +5,7 @@
 // object table are static per scene, so they are turned into straight-line CUDA with the (%.6f-quantised, sscanf-parsed)
 // transforms as immediates instead of being interpreted per sample.
 #include "host_internal.h"
+#include <elf.h>
 #include "scene_module_src.inc"     // generated: kScenePrelude, kSceneParams, kSceneKernels (raw strings)
 
 using namespace dcsg_host;
@@ -160,6 +161,44 @@ std::string dot_expression(const float a[3], int lastAxis, const std::string d[3
 // !(|d| >= 2^-60) when the core is a single product d * a with 2^-40 <= |a| (it then cannot be or round to zero; objects
 // that share an axis and an offset share the test), or core == 0 tested on the value itself when two terms remain.
 // Design1: 66 FFMAs per evaluation become 12 compares.
+// One local coordinate (axis vector k of object o) in the fast copy's form, over the differences d[]: `expr`, and what guards
+// it when zero terms were dropped -- `testAxis` >= 0: |d[testAxis]| >= 2^-60 (a single product); `testCore`: |expr| > 0.
+// elided = false: the exact form, dot_expression(.., lastAxis, d), no test.
+struct FastCoordinate {
+    std::string expr;
+    bool elided = false, testCore = false;
+    int testAxis = -1;
+};
+FastCoordinate fast_coordinate(const Scene& sc, int o, int k, int lastAxis, const std::string d[3]) {
+    const float (*axes[3])[3] = {&sc.right[o], &sc.up[o], &sc.forward[o]};
+    const float* a = *axes[k];
+    FastCoordinate fc;
+    std::vector<int> rest, zeros;
+    for (int c = 0; c < 3; c++) (is_zero_coefficient(a[c]) ? zeros : rest).push_back(c);
+    bool elide = !zeros.empty() && !rest.empty();
+    for (int c : zeros) elide = elide && fabsf(sc.position[o][c]) < 0x1p100f;
+    if (elide && rest.size() == 1) elide = fabsf(a[rest[0]]) >= 0x1p-40f;       // NaN coefficients fail this too
+    if (!elide) {
+        fc.expr = dot_expression(a, lastAxis, d);
+        return fc;
+    }
+    fc.elided = true;
+    auto product = [&](int c) { return d[c] + " * " + float_literal(a[c]); };
+    if (rest.size() == 1) {
+        fc.expr = product(rest[0]);
+        fc.testAxis = rest[0];
+    } else {
+        // two non-zero terms: the reference's sum of the two products (dot_expression without the zero term)
+        const int i = rest[0], j = rest[1];
+        auto fused = [&](int c, const std::string& acc) { return "__fmaf_rn(" + d[c] + ", " + float_literal(a[c]) + ", " + acc + ")"; };
+        if (is_unit_coefficient(a[i])) fc.expr = fused(i, product(j));
+        else if (is_unit_coefficient(a[j])) fc.expr = fused(j, product(i));
+        else fc.expr = "(" + product(i) + " + " + product(j) + ")";
+        fc.testCore = true;
+    }
+    return fc;
+}
+
 bool generate_primary_sdf(const Scene& sc, bool rowVariant, bool fast, std::string& out, std::string& err) {
     std::set<std::pair<int, uint32_t>> tested;          // (axis, position bits) whose difference already has its magnitude test
     bool anyElided = false;
@@ -186,34 +225,16 @@ bool generate_primary_sdf(const Scene& sc, bool rowVariant, bool fast, std::stri
             const char* names[3] = {"dcsg_la", "dcsg_lb", "dcsg_lc"};
             const std::string dnames[3] = {"dcsg_dx", "dcsg_dy", "dcsg_dz"};
             for (int k = 0; k < 3; k++) {
-                const float* a = *axes[k];
-                std::vector<int> rest, zeros;
-                for (int c = 0; c < 3; c++) (is_zero_coefficient(a[c]) ? zeros : rest).push_back(c);
-                bool elide = fast && !zeros.empty() && !rest.empty();
-                for (int c : zeros) elide = elide && fabsf(sc.position[o][c]) < 0x1p100f;
-                if (elide && rest.size() == 1) elide = fabsf(a[rest[0]]) >= 0x1p-40f;       // NaN coefficients fail this too
-                if (!elide) {
-                    body += "        const float " + std::string(names[k]) + " = " + dot_expression(a, rowVariant ? 0 : -1, dnames) + ";\n";
+                if (!fast) {
+                    body += "        const float " + std::string(names[k]) + " = " + dot_expression(*axes[k], rowVariant ? 0 : -1, dnames) + ";\n";
                     continue;
                 }
-                anyElided = true;
-                if (rest.size() == 1) {
-                    const int c = rest[0];
-                    body += "        const float " + std::string(names[k]) + " = " + dnames[c] + " * " + float_literal(a[c]) + ";\n";
-                    if (tested.insert({c, float_bits(sc.position[o][c])}).second)
-                        body += "        DCSG_BAD_UNLESS_ABS_GE(" + dnames[c] + ", 8.6736173798840355e-19f);\n";      // 2^-60
-                } else {
-                    // two non-zero terms: the reference's sum of the two products (dot_expression without the zero term)
-                    const int i = rest[0], j = rest[1];
-                    std::string core;
-                    auto product = [&](int c) { return dnames[c] + " * " + float_literal(a[c]); };
-                    auto fused = [&](int c, const std::string& acc) { return "__fmaf_rn(" + dnames[c] + ", " + float_literal(a[c]) + ", " + acc + ")"; };
-                    if (is_unit_coefficient(a[i])) core = fused(i, product(j));
-                    else if (is_unit_coefficient(a[j])) core = fused(j, product(i));
-                    else core = "(" + product(i) + " + " + product(j) + ")";
-                    body += "        const float " + std::string(names[k]) + " = " + core + ";\n";
-                    body += "        DCSG_BAD_UNLESS_ABS_GT0(" + std::string(names[k]) + ");\n";
-                }
+                const FastCoordinate fc = fast_coordinate(sc, o, k, rowVariant ? 0 : -1, dnames);
+                body += "        const float " + std::string(names[k]) + " = " + fc.expr + ";\n";
+                anyElided = anyElided || fc.elided;
+                if (fc.testAxis >= 0 && tested.insert({fc.testAxis, float_bits(sc.position[o][fc.testAxis])}).second)
+                    body += "        DCSG_BAD_UNLESS_ABS_GE(" + dnames[fc.testAxis] + ", 8.6736173798840355e-19f);\n";      // 2^-60
+                if (fc.testCore) body += "        DCSG_BAD_UNLESS_ABS_GT0(" + std::string(names[k]) + ");\n";
             }
             body += format("        dcsg_s%d = sdf_bank(float3(dcsg_la, dcsg_lb, dcsg_lc), (unsigned char)%d);\n    }\n", dst, lhs & 0xff);
         } break;
@@ -331,6 +352,116 @@ bool generate_primary_sdf7(const Scene& sc, std::string& out, std::string& err) 
     return true;
 }
 
+// The taps of a normal along ONE world axis, for namespace dcsg_fast: the fast copy's evaluations at v + e and v - e on that
+// axis (and at v itself when `centre`), as one straight-line function, object-major.  For every IMPORT the differences and
+// local coordinates of its evaluations are formed next to each other, each distinct one once, the varying axis' terms last;
+// then sdf_bank runs once per evaluation, and the compiler's value numbering shares inside the inlined brush whatever depends
+// on the unchanged coordinates only.  For an axis-aligned object a local coordinate is one product (v.c - o.c) * a of ONE
+// world coordinate, so a tap along x leaves every y- and z-dependent value of every object unchanged.
+//
+// Three coordinate variants are enough.  The reference's taps are v + (e,0,0) and v - (e,0,0): the unchanged coordinates of
+// a plus tap are v.c + 0.0f, those of a minus tap and of the centre v.c.  They differ only where v.c is -0 (+0 then), and a
+// NaN may come out of the addition with other bits.  So every function also tests its own axis' coordinate, !(|v.c| > 0):
+// with the flag of a whole round (x, y and z functions) down no coordinate is +-0 or NaN, v.c + 0.0f and v.c are the same
+// bits, and the seven evaluations only need v.c, v.c + e and v.c - e.  The other tests are the single-evaluation form's
+// (generate_primary_sdf, fast): |coordinate| < 2^120 for every coordinate value an evaluation uses (each function tests its
+// axis' three values: together they cover all of them), and the magnitude tests of the elided transform terms, each distinct
+// one emitted once.  The flag is the union of all of them, so where it stays down each value is the single-evaluation fast
+// form's value at that tap, which is the exact copy's.  A vertex exactly on a coordinate plane already fails the |d| >= 2^-60
+// test of an object centred there, so on such scenes the zero test flags nothing new.
+// out[] order: +axis, -axis, centre.
+bool generate_primary_sdf_axis(const Scene& sc, int axis, bool centre, std::string& out, std::string& err) {
+    const char* comp[3] = {"x", "y", "z"};
+    // coordinate variables: dcsg_c<axis>0 = v.c, dcsg_c<axis>p = v.c + e, dcsg_c<axis>m = v.c - e
+    auto coordinate = [&](int k, char variant) { return format("dcsg_c%s%c", comp[k], k == axis ? variant : '0'); };
+    std::vector<std::array<std::string, 3>> evals;
+    for (char variant : centre ? std::string("pm0") : std::string("pm")) evals.push_back({coordinate(0, variant), coordinate(1, variant), coordinate(2, variant)});
+    const int n = (int)evals.size();
+    std::set<std::pair<std::string, uint32_t>> tested;     // (coordinate variable, position bits) whose difference has its test
+    bool anyElided = false;
+    bool used[DCSG_STACK_SLOTS] = {false};
+    auto slot_ok = [&](int s) { return s >= 0 && s < DCSG_STACK_SLOTS; };
+    std::string body;
+    for (int i = 0; i < sc.num_steps; i++) {
+        const int op = sc.steps[i][0], lhs = sc.steps[i][1], rhs = sc.steps[i][2], dst = sc.steps[i][3];
+        switch (op) {
+        case 0: {   // IMPORT
+            if (rhs < 0 || rhs >= sc.num_objects || !slot_ok(dst)) { err = format("buildprocedure.txt command %d: bad IMPORT", i); return false; }
+            used[dst] = true;
+            const int o = rhs;
+            body += format("    {   // object %d, brush %d -> slot %d, all evaluations of the function\n", o, lhs, dst);
+            std::map<std::string, std::string> diff, local;     // coordinate variable -> difference; expression -> local coordinate
+            auto difference = [&](const std::string& c, int k) {
+                auto it = diff.find(c);
+                if (it != diff.end()) return it->second;
+                const std::string name = "dcsg_d" + c.substr(6);
+                if (float_bits(sc.position[o][k]) == 0u) body += "        const float " + name + " = " + c + ";\n";
+                else body += "        const float " + name + " = " + c + " - " + float_literal(sc.position[o][k]) + ";\n";
+                return diff[c] = name;
+            };
+            for (int k : {(axis + 1) % 3, (axis + 2) % 3, axis})        // the varying axis last
+                for (const auto& e : evals) difference(e[k], k);
+            std::vector<std::array<std::string, 3>> locals(n);
+            for (int k = 0; k < 3; k++)
+                for (int t = 0; t < n; t++) {
+                    const std::string d[3] = {diff[evals[t][0]], diff[evals[t][1]], diff[evals[t][2]]};
+                    const FastCoordinate fc = fast_coordinate(sc, o, k, axis, d);
+                    anyElided = anyElided || fc.elided;
+                    auto it = local.find(fc.expr);
+                    if (it != local.end()) { locals[t][k] = it->second; continue; }
+                    const std::string name = format("dcsg_l%d_%d", k, (int)local.size());
+                    local[fc.expr] = locals[t][k] = name;
+                    body += "        const float " + name + " = " + fc.expr + ";\n";
+                    if (fc.testAxis >= 0 && tested.insert({evals[t][fc.testAxis], float_bits(sc.position[o][fc.testAxis])}).second)
+                        body += "        DCSG_BAD_UNLESS_ABS_GE(" + d[fc.testAxis] + ", 8.6736173798840355e-19f);\n";      // 2^-60
+                    if (fc.testCore) body += "        DCSG_BAD_UNLESS_ABS_GT0(" + name + ");\n";
+                }
+            for (int t = 0; t < n; t++)
+                body += format("        dcsg_s%d_%d = sdf_bank(float3(%s, %s, %s), (unsigned char)%d);\n", dst, t, locals[t][0].c_str(),
+                               locals[t][1].c_str(), locals[t][2].c_str(), lhs & 0xff);
+            body += "    }\n";
+        } break;
+        case 1:     // EXPORT
+            if (!slot_ok(lhs)) { err = format("buildprocedure.txt command %d: bad EXPORT", i); return false; }
+            used[lhs] = true;
+            for (int t = 0; t < n; t++) body += format("    dcsg_out[%d] = dcsg_s%d_%d;\n", t, lhs, t);
+            break;
+        case 2: case 3:
+            if (!slot_ok(lhs) || !slot_ok(rhs) || !slot_ok(dst)) { err = format("buildprocedure.txt command %d: bad slot", i); return false; }
+            used[lhs] = used[rhs] = used[dst] = true;
+            for (int t = 0; t < n; t++)
+                body += format("    dcsg_s%d_%d = %s(dcsg_s%d_%d,dcsg_s%d_%d);\n", dst, t, op == 2 ? "T_min" : "T_max", lhs, t, rhs, t);
+            break;
+        case 4: case 5:
+            if (!slot_ok(lhs) || !slot_ok(dst)) { err = format("buildprocedure.txt command %d: bad slot", i); return false; }
+            used[lhs] = used[dst] = true;
+            for (int t = 0; t < n; t++) body += format("    dcsg_s%d_%d = %sdcsg_s%d_%d;\n", dst, t, op == 4 ? "-" : "", lhs, t);
+            break;
+        default:
+            break;  // unknown opcodes fall through the reference's switch without effect
+        }
+    }
+    const std::string c = comp[axis];
+    out = format("\n// ---- generated by dcsg_build: the %s-taps of a normal%s, see generate_primary_sdf_axis ----\n", c.c_str(),
+                 centre ? " and the centre" : "") +
+          format("__device__ __forceinline__ void dcsg_primary_sdf_%s%s(float3 dcsg_v, float dcsg_e, float (&dcsg_out)[%d], bool& dcsg_inexact_out) {\n",
+                 c.c_str(), centre ? "c" : "", n) +
+          "    DCSG_BAD_DECLARE();\n";
+    for (int k = 0; k < 3; k++) out += format("    const float dcsg_c%s0 = dcsg_v.%s;\n", comp[k], comp[k]);
+    out += format("    const float dcsg_c%sp = dcsg_v.%s + dcsg_e;\n", c.c_str(), c.c_str());
+    out += format("    const float dcsg_c%sm = dcsg_v.%s - dcsg_e;\n", c.c_str(), c.c_str());
+    out += format("    DCSG_BAD_UNLESS_ABS_GT0(dcsg_c%s0);\n", c.c_str());
+    if (anyElided)
+        for (const char* v : {"0", "p", "m"}) out += format("    DCSG_BAD_UNLESS_ABS_LT(dcsg_c%s%s, 1.329227995784916e+36f);\n", c.c_str(), v);    // 2^120
+    for (int t = 0; t < n; t++) out += format("    dcsg_out[%d] = MAX_DISTANCE;\n", t);
+    for (int s = 0; s < DCSG_STACK_SLOTS; s++)
+        if (used[s])
+            for (int t = 0; t < n; t++) out += format("    float dcsg_s%d_%d = 0.0f;\n", s, t);
+    out += body;
+    out += "    DCSG_BAD_COMMIT(dcsg_inexact_out);\n}\n";
+    return true;
+}
+
 // The object loop of the preview's shade (reference k1.cl:300-325) with the object table as immediates: every object's
 // own SDF is evaluated at the hit point; the LAST object within SDF_EPSILON * TOLERANCE_FACTOR_MATERIAL decides the
 // material (k1.cl:318-321), whose shader then receives the global point, that object's local point and the normal.
@@ -365,14 +496,23 @@ bool scene_wants_fast_path(const Scene& sc) {
     return sc.private_words == 0 && !(off && off[0] == '1');
 }
 
-std::string assemble_source(const Scene& sc, bool fastPath, std::string& err, bool flagInShared) {
-    std::string gen, genRow, gen7, genFast;
+std::string assemble_source(const Scene& sc, bool fastPath, std::string& err, bool flagInShared, bool tapAxes) {
+    std::string gen, genRow, gen7, genFast, genAxes;
     if (!generate_primary_sdf(sc, false, false, gen, err) || !generate_primary_sdf(sc, true, false, genRow, err) ||
         !generate_primary_sdf7(sc, gen7, err) || (fastPath && !generate_primary_sdf(sc, false, true, genFast, err)))
         return std::string();
+    if (fastPath) {
+        // per-axis forms: x with the centre (projection), x without it (normals alone), y, z
+        for (int f = 0; f < 4; f++) {
+            std::string one;
+            if (!generate_primary_sdf_axis(sc, f == 0 ? 0 : f - 1, f == 0, one, err)) return std::string();
+            genAxes += one;
+        }
+    }
     std::string src;
     src.reserve(1 << 17);
     src += format("#define DCSG_FAST_PATH %d\n", fastPath ? 1 : 0);
+    if (fastPath && tapAxes) src += "#define DCSG_TAP_AXES 1\n";
     if (flagInShared) src += "#define DCSG_FLAG_PRED 0\n";
     src += kScenePrelude;
     src += "\nnamespace dcsg_exact {\n#define DCSG_SQRT_F32(x) ::sqrtf(x)\n";
@@ -396,6 +536,12 @@ std::string assemble_source(const Scene& sc, bool fastPath, std::string& err, bo
     src += generate_shade_objects(sc);
     src += "}  // namespace dcsg_exact\n";
     if (fastPath) {
+        // The per-axis forms sit in a block of their own in front of the fast copy's scene text, so that block holds the same
+        // two texts as the exact copy's.  They reach its brushes through a declaration of sdf_bank, whose signature
+        // scenecompiler emits (a scene whose text does not match fails to compile here, and compile_scene keeps the loop).
+        src += "\nnamespace dcsg_fast {\n__device__ float sdf_bank(float3 v, unsigned char shape_id);\n";
+        src += genAxes;
+        src += "}  // namespace dcsg_fast\n";
         src += "\nnamespace dcsg_fast {\n// ---- scene.cu once more, against the checked fast forms ----\n";
         src += user;
         src += genFast;
@@ -406,11 +552,106 @@ std::string assemble_source(const Scene& sc, bool fastPath, std::string& err, bo
 
 // Compile the scene: with the checked fast copy when the design allows it, and -- should user text that compiles once
 // not compile twice (it is pasted into two namespaces) -- exact-only, with a note in the log.
+bool kernel_footprint(const std::vector<char>& cubin, const char* kernel, KernelFootprint& fp) {
+    fp = KernelFootprint();
+    const char* base = cubin.data();
+    const size_t size = cubin.size();
+    if (size < sizeof(Elf64_Ehdr) || memcmp(base, ELFMAG, SELFMAG) != 0 || base[EI_CLASS] != ELFCLASS64) return false;
+    Elf64_Ehdr eh;
+    memcpy(&eh, base, sizeof(eh));
+    if (eh.e_shentsize != sizeof(Elf64_Shdr) || eh.e_shoff + (uint64_t)eh.e_shnum * sizeof(Elf64_Shdr) > size || eh.e_shstrndx >= eh.e_shnum) return false;
+    std::vector<Elf64_Shdr> sh(eh.e_shnum);
+    memcpy(sh.data(), base + eh.e_shoff, eh.e_shnum * sizeof(Elf64_Shdr));
+    for (const Elf64_Shdr& s : sh)
+        if (s.sh_type != SHT_NOBITS && s.sh_offset + s.sh_size > size) return false;
+    auto cstr = [&](const Elf64_Shdr& table, uint32_t at) -> std::string {
+        if (at >= table.sh_size) return std::string();
+        const char* p = base + table.sh_offset + at;
+        return std::string(p, strnlen(p, table.sh_size - at));
+    };
+    const std::string textName = std::string(".text.") + kernel;
+    int text = -1, symtab = -1, info = -1;
+    for (int i = 0; i < (int)sh.size(); i++) {
+        const std::string name = cstr(sh[eh.e_shstrndx], sh[i].sh_name);
+        if (name == textName) text = i;
+        else if (sh[i].sh_type == SHT_SYMTAB) symtab = i;
+        else if (name == ".nv.info") info = i;
+    }
+    if (text < 0 || symtab < 0 || info < 0 || sh[symtab].sh_link >= sh.size() || sh[symtab].sh_entsize != sizeof(Elf64_Sym)) return false;
+    fp.textBytes = sh[text].sh_size;
+    // the kernel's symbol, and every function whose code lies in its text section (callees that are not inlined)
+    std::set<uint32_t> inText;
+    uint32_t kernelSym = UINT32_MAX;
+    for (uint64_t off = 0; off + sizeof(Elf64_Sym) <= sh[symtab].sh_size; off += sizeof(Elf64_Sym)) {
+        Elf64_Sym sym;
+        memcpy(&sym, base + sh[symtab].sh_offset + off, sizeof(sym));
+        const uint32_t idx = (uint32_t)(off / sizeof(Elf64_Sym));
+        if (sym.st_shndx != text || ELF64_ST_TYPE(sym.st_info) != STT_FUNC) continue;
+        inText.insert(idx);
+        if (cstr(sh[sh[symtab].sh_link], sym.st_name) == kernel) kernelSym = idx;
+    }
+    if (kernelSym == UINT32_MAX) return false;
+    // .nv.info: records of {u8 format, u8 attribute, u16 value-or-size}; format 4 (EIFMT_SVAL) carries `size` bytes after
+    // the header.  EIATTR_REGCOUNT (0x2f) and EIATTR_FRAME_SIZE (0x11) are SVALs of {u32 symbol, u32 value}.
+    const char* p = base + sh[info].sh_offset;
+    const char* end = p + sh[info].sh_size;
+    while (p + 4 <= end) {
+        const uint8_t format = (uint8_t)p[0], attribute = (uint8_t)p[1];
+        uint16_t value;
+        memcpy(&value, p + 2, 2);
+        const uint32_t payload = format == 4 ? value : 0u;
+        if (p + 4 + payload > end) return false;
+        if (format == 4 && payload >= 8 && (attribute == 0x2f || attribute == 0x11)) {
+            uint32_t sym, v;
+            memcpy(&sym, p + 4, 4);
+            memcpy(&v, p + 8, 4);
+            if (attribute == 0x2f && sym == kernelSym) fp.registers = (int)v;
+            if (attribute == 0x11 && inText.count(sym)) fp.frameBytes = std::max(fp.frameBytes, v);
+        }
+        p += 4 + payload;
+    }
+    return fp.registers >= 0;
+}
+
+// The per-axis tap form earns its place when dcsg_k_project stays within 64 registers (four resident blocks of 256 threads:
+// __launch_bounds__ in scene_kernels.cuh), without local memory, and with text small enough for the instruction cache.
+// The projection kernel on sm_100a, rolled loop -> per-axis form (DESIGN.md 3b): Design1 23.4 -> 36.6 KiB of code at 64
+// registers, projection 7.83 -> 6.48 ms at 1024^3 on a B200; the Hilbert design (design2) 37.2 -> 108.1 KiB, 12.75 -> 15.52 ms
+// (instruction cache misses); synth64 22.6 -> 38.8 KiB; the stress scene and the random* scenes spill at 64 registers.
+static const uint64_t kAxisTextLimit = 64 * 1024;
+
+// Empty when the per-axis form of this cubin fits the budget, else why not.
+static std::string axis_form_misfit(const std::vector<char>& cubin) {
+    KernelFootprint fp;
+    if (!kernel_footprint(cubin, "dcsg_k_project", fp)) return "the footprint of dcsg_k_project could not be read from the cubin";
+    if (fp.registers > 64) return format("dcsg_k_project needs %d registers (budget 64)", fp.registers);
+    if (fp.frameBytes > 0) return format("dcsg_k_project has a stack frame of %u bytes (local memory)", fp.frameBytes);
+    if (fp.textBytes > kAxisTextLimit)
+        return format("dcsg_k_project is %.1f KiB of code (limit %.0f KiB)", fp.textBytes / 1024.0, kAxisTextLimit / 1024.0);
+    return std::string();
+}
+
+// DCSG_TAP_FORM=loop / axis forces the tap form of the fast copy (to compare the two); unset, the footprint decides.
 bool compile_scene(const Scene& sc, std::vector<char>& cubin, std::string& log, std::string& err, bool exactOnly) {
     if (!exactOnly && scene_wants_fast_path(sc)) {
+        const char* form = getenv("DCSG_TAP_FORM");
+        const bool loopForced = form && strcmp(form, "loop") == 0, axisForced = form && strcmp(form, "axis") == 0;
+        std::string loopNote;
+        if (!loopForced) {
+            const std::string src = assemble_source(sc, true, err, false, true);
+            if (src.empty()) return false;
+            std::string misfit;
+            if (compile_source(src, cubin, log)) {
+                misfit = axis_form_misfit(cubin);
+                if (misfit.empty() || axisForced) return true;
+            } else {
+                misfit = "the per-axis form did not compile";
+            }
+            loopNote = "[dcsg] the normals keep the rolled tap loop: " + misfit + "\n";
+        }
         const std::string src = assemble_source(sc, true, err);
         if (src.empty()) return false;
-        if (compile_source(src, cubin, log)) return true;
+        if (compile_source(src, cubin, log)) { log = loopNote + log; return true; }
         // The fast copy keeps its flag in a PTX predicate register of the kernel (scene_prelude.cuh), which needs every
         // function of the copy inlined into the kernels; text that does not inline still builds with the flag in shared memory.
         std::string sharedLog;

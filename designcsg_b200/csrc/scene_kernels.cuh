@@ -52,8 +52,9 @@ DCSG_DEV float dcsg_sdf(float3 q) { return dcsg_exact::dcsg_primary_sdf(q); }
 // normal + value at one point.  Reference get_normal (k2.cl:149-179): six taps at +-NORMAL_EPSILON
 // (a double literal narrowed to float when the tap vectors are built), differences in float, the
 // 1/(2e) scale in double (`1.0/twoE*Dx`), then normalize.  The seven evaluations (six taps and,
-// optionally, the centre) run through ONE inlined copy of the SDF inside a rolled loop, which keeps
-// the instruction footprint of heavy scenes inside the instruction cache.
+// optionally, the centre) run through the fast copy's per-axis straight-line forms where the scene's
+// projection kernel fits their budget (compile_scene), else through ONE inlined copy of the SDF inside
+// a rolled loop, which keeps the instruction footprint of heavy scenes inside the instruction cache.
 // ---------------------------------------------------------------------------------------------
 #ifndef DCSG_TAPS_SHARED
 // 1 = dcsg_primary_sdf7: the seven evaluations as one straight-line function whose taps share the transform
@@ -62,6 +63,11 @@ DCSG_DEV float dcsg_sdf(float3 q) { return dcsg_exact::dcsg_primary_sdf(q); }
 // on the Hilbert design (instruction footprint) -- so the loop stays the default; -DDCSG_TAPS_SHARED=1 through
 // DCSG_NVRTC_EXTRA selects the other form (tests pass with either).
 #define DCSG_TAPS_SHARED 0
+#endif
+#ifndef DCSG_TAP_AXES
+// 1 = the fast copy's taps through the per-axis forms (dcsg_fast::dcsg_primary_sdf_x / _y / _z), chosen per scene by
+// compile_scene; 0 = rolled loop over one inlined copy
+#define DCSG_TAP_AXES 0
 #endif
 // Rolled tap loop without per-iteration selects: tap k is v + dcsg_tap_offset[k] and its value goes to a per-thread
 // column of shared memory.  The reference builds the taps as v + (e,0,0), v - (e,0,0), ... (k2.cl:155-166); in IEEE
@@ -87,6 +93,55 @@ DCSG_DEV float3 dcsg_normal_and_sdf_mode(float3 v, float& centre, bool& flagged)
         float f[7];
         dcsg_exact::dcsg_primary_sdf7(v, DCSG_TAP_E, f);         // the centre's value is dead code when kWithCentre is false
         f0 = f[0]; f1 = f[1]; f2 = f[2]; f3 = f[3]; f4 = f[4]; f5 = f[5]; f6 = f[6];
+    }
+#elif DCSG_FAST_PATH && DCSG_TAP_AXES
+    // The fast copy through the per-axis forms (host_scene.cu, generate_primary_sdf_axis): straight-line code in which the
+    // taps of an axis share the unchanged coordinates' work, values in registers.  Their tests include every test of the
+    // seven single evaluations, plus one the loop does not need (a coordinate of exactly +-0 or NaN).  So a flagged round
+    // runs the rolled loop of the fast copy next, and only if that flags too does it go to the exact copy (mode 0) or
+    // the caller (mode 1): a round is flagged exactly when the rolled loop would flag it, with the same values.
+    {
+        float* const mine = dcsg_tap_value + threadIdx.x;
+        bool exact = kMode == 2;
+        if (kMode != 2) {
+            bool inexact = false;
+            float tx[kWithCentre ? 3 : 2], ty[2], tz[2];
+            if constexpr (kWithCentre) dcsg_fast::dcsg_primary_sdf_xc(v, DCSG_TAP_E, tx, inexact);
+            else dcsg_fast::dcsg_primary_sdf_x(v, DCSG_TAP_E, tx, inexact);
+            dcsg_fast::dcsg_primary_sdf_y(v, DCSG_TAP_E, ty, inexact);
+            dcsg_fast::dcsg_primary_sdf_z(v, DCSG_TAP_E, tz, inexact);
+            f0 = tx[0]; f1 = tx[1]; f2 = ty[0]; f3 = ty[1]; f4 = tz[0]; f5 = tz[1];
+            if constexpr (kWithCentre) f6 = tx[2];
+            if (inexact | dcsg_flag_take()) {                      // one test for the round
+                bool again = false;
+#pragma unroll 1
+                for (int k = 0; k < (kWithCentre ? 7 : 6); ++k) {
+                    const float3 q = float3(v.x + dcsg_tap_offset[k][0], v.y + dcsg_tap_offset[k][1], v.z + dcsg_tap_offset[k][2]);
+                    mine[k * DCSG_BLOCK] = dcsg_fast::dcsg_primary_sdf(q, again);
+                }
+                if (again | dcsg_flag_take()) {
+                    if (kMode == 1) {
+                        flagged = true;
+                    } else {                                       // all seven are evaluated again
+                        dcsg_exact_rounds[threadIdx.x] += 1u;
+                        exact = true;
+                    }
+                }
+                if (!flagged && !exact) {
+                    f0 = mine[0 * DCSG_BLOCK]; f1 = mine[1 * DCSG_BLOCK]; f2 = mine[2 * DCSG_BLOCK];
+                    f3 = mine[3 * DCSG_BLOCK]; f4 = mine[4 * DCSG_BLOCK]; f5 = mine[5 * DCSG_BLOCK];
+                    if (kWithCentre) f6 = mine[6 * DCSG_BLOCK];
+                }
+            }
+        }
+        if (exact) {
+#pragma unroll 1
+            for (int k = 0; k < (kWithCentre ? 7 : 6); ++k)
+                mine[k * DCSG_BLOCK] = dcsg_sdf_exact_call(v.x + dcsg_tap_offset[k][0], v.y + dcsg_tap_offset[k][1], v.z + dcsg_tap_offset[k][2]);
+            f0 = mine[0 * DCSG_BLOCK]; f1 = mine[1 * DCSG_BLOCK]; f2 = mine[2 * DCSG_BLOCK];
+            f3 = mine[3 * DCSG_BLOCK]; f4 = mine[4 * DCSG_BLOCK]; f5 = mine[5 * DCSG_BLOCK];
+            if (kWithCentre) f6 = mine[6 * DCSG_BLOCK];
+        }
     }
 #else
     {
@@ -892,7 +947,14 @@ DCSG_DEV void dcsg_project_phase(const dcsg_project_args& a, unsigned& rounds) {
     }
 }
 
-extern "C" __global__ void __launch_bounds__(DCSG_BLOCK)
+// the per-axis form holds a tap round's values in registers: at most 64 of them, four resident blocks per SM (compile_scene
+// checks the result and keeps the rolled loop for a scene whose kernel does not fit)
+#if DCSG_FAST_PATH && DCSG_TAP_AXES
+#define DCSG_PROJECT_BOUNDS __launch_bounds__(DCSG_BLOCK, 4)
+#else
+#define DCSG_PROJECT_BOUNDS __launch_bounds__(DCSG_BLOCK)
+#endif
+extern "C" __global__ void DCSG_PROJECT_BOUNDS
 dcsg_k_project(const dcsg_project_args a, dcsg_u64* __restrict__ stats) {
     dcsg_enter();
     const unsigned lane = threadIdx.x & 31u;
