@@ -2,6 +2,9 @@
 
     python -m designcsg_b200 compile DESIGN.py SCENE_DIR              design script -> scene files ("Run")
     python -m designcsg_b200 export  SCENE_DIR|DESIGN.py [--level L] [--ply P] [--stl S] [--normals]
+    python -m designcsg_b200 export  SCENE_DIR|DESIGN.py --ply-indexed P [--normals] [--level L]
+                                                                       indexed binary PLY (shared float vertices, optional
+                                                                       normals; not the reference's format)
     torchrun --nproc-per-node G -m designcsg_b200 export ...          z-slab sharded over G GPUs (dcsg_export_sharded; the
                                                                        same export from a C host: tools/dcsg_mgpu.c)
 """
@@ -45,6 +48,16 @@ def cmd_export(args):
     world = int(os.environ.get("WORLD_SIZE", "1"))
     rank = int(os.environ.get("RANK", "0"))
     local = int(os.environ.get("LOCAL_RANK", "0"))
+    if args.ply_indexed:
+        # checked before anything is built or a device is touched
+        if args.ply or args.stl:
+            raise SystemExit("--ply-indexed cannot be combined with --ply / --stl: the two exports would project the mesh twice, "
+                             "and the indexed file welds an adaptive mesh before its projection; run them separately")
+        if args.no_retopologize:
+            raise SystemExit("--ply-indexed re-encodes the reference's export, which always retopologizes: drop --no-retopologize")
+        if world > 1 and not args.level:
+            raise SystemExit("--ply-indexed on several GPUs needs --level L (a uniform lattice): the weld of an adaptive mesh "
+                             "spans the GPUs' slabs")
     build.build()                       # serialised across the ranks of a node by a file lock; the first one compiles
     scene = _scene_dir(args.scene)
     cfg = _export_config(scene)
@@ -62,7 +75,12 @@ def cmd_export(args):
     ctx.build(scene)
     t_build = time.perf_counter() - t0
     report = {"scene": scene, "octree_levels": [lo, hi, level], "gd_steps": steps, "gpus": world, "build_s": t_build}
-    if world == 1:
+    if world == 1 and args.ply_indexed:
+        t1 = time.perf_counter()
+        rep = ctx.export_indexed(scene, args.level, args.ply_indexed, normals=args.normals)
+        report.update(triangles=int(rep.num_triangles), vertices=int(rep.num_vertices), box=[float(v) for v in rep.box],
+                      export_s=time.perf_counter() - t1, project_and_write_ms=float(rep.write_ms))
+    elif world == 1:
         box = ctx.bbox(search)
         report["box"] = [float(v) for v in box]
         pipelined = not args.normals                       # projection pipelined with formatting, D2H and the file writes
@@ -83,7 +101,7 @@ def cmd_export(args):
         import torch
         import torch.distributed as dist
         from . import distributed as D
-        if args.normals:
+        if args.normals and not args.ply_indexed:
             raise SystemExit("--normals has no effect on the files (the reference's writers store no normals) and is not "
                              "supported by the sharded export; drop it or run on one GPU")
         if not cfg:
@@ -92,7 +110,10 @@ def cmd_export(args):
         dist.init_process_group("nccl", device_id=torch.device("cuda", local))
         comm = D.create_comm(ctx)       # from here on everything collective happens inside libdcsg
         t1 = time.perf_counter()
-        rep = comm.export(scene, args.level, args.stl, args.ply)
+        if args.ply_indexed:
+            rep = comm.export_indexed(scene, args.level, args.ply_indexed, normals=args.normals)
+        else:
+            rep = comm.export(scene, args.level, args.stl, args.ply)
         report.update(triangles=int(rep.num_triangles), vertices=int(rep.num_vertices), box=[float(v) for v in rep.box],
                       export_s=time.perf_counter() - t1, search_ms=float(rep.bbox_ms), project_and_write_ms=float(rep.write_ms))
         comm.close()
@@ -117,6 +138,8 @@ def main():
     e.add_argument("--no-retopologize", action="store_true", help="skip cms::retopologize (identity for uniform lattices)")
     e.add_argument("--ply")
     e.add_argument("--stl")
+    e.add_argument("--ply-indexed", help="write an indexed binary PLY instead (shared float vertices; with --normals the "
+                   "projection's normals too) -- a format beyond the reference's")
     e.add_argument("--normals", action="store_true")
     e.set_defaults(fn=cmd_export)
     args = ap.parse_args()

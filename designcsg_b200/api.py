@@ -65,6 +65,8 @@ PROGRESS_STATES = ("IDLE", "ESTIMATING_BOUNDING_BOX", "PERFORMING_CMS", "RETOPOL
                    "WRITING_PLY", "COMPLETE")                   # dcsg.h DCSG_PROGRESS_*, reference DesignCSG.cpp:603-614
 PROGRESS_FN = ctypes.CFUNCTYPE(None, ctypes.c_void_p, ctypes.c_int, ctypes.c_uint64, ctypes.c_uint64)
 
+PLY_NORMALS = 1                                                 # dcsg.h DCSG_PLY_NORMALS
+
 _lib = None
 
 
@@ -134,6 +136,10 @@ def load_library():
     lib.dcsg_export_sharded.argtypes = [vp, vp, cp, ci, cp, cp, ctypes.POINTER(ExportReport)]
     lib.dcsg_project.argtypes = [vp, ctypes.POINTER(MeshStruct), ci, ci]
     lib.dcsg_plan_slabs.argtypes = [vp, _f32p, ci, ci, ci, ctypes.POINTER(ci)]
+    lib.dcsg_mesh_weld.argtypes = [vp, ctypes.POINTER(MeshStruct)]
+    lib.dcsg_write_ply_indexed.argtypes = [vp, ctypes.POINTER(MeshStruct), ci, cp]
+    lib.dcsg_export_indexed.argtypes = [vp, cp, ci, ci, cp, ctypes.POINTER(ExportReport)]
+    lib.dcsg_export_sharded_indexed.argtypes = [vp, vp, cp, ci, ci, cp, ctypes.POINTER(ExportReport)]
     _lib = lib
     return lib
 
@@ -290,6 +296,16 @@ class Mesh:
 
     def write_ply(self, path):
         self._ctx._check(self._ctx.lib.dcsg_write_ply(self._ctx.h, ctypes.byref(self.c), path.encode()))
+
+    def weld(self):
+        """dcsg_mesh_weld: merge vertices with bit-identical positions (numbered by first occurrence), renumber the triangles.
+        A lattice mesh comes back unchanged.  The host arrays are refreshed when the mesh was copied to the host."""
+        self._ctx._check(self._ctx.lib.dcsg_mesh_weld(self._ctx.h, ctypes.byref(self.c)))
+
+    def write_ply_indexed(self, path, normals=False):
+        """dcsg_write_ply_indexed: binary PLY with shared float vertices (and the mesh's normals) -- not the reference's format."""
+        self._ctx._check(self._ctx.lib.dcsg_write_ply_indexed(self._ctx.h, ctypes.byref(self.c), PLY_NORMALS if normals else 0,
+                                                              path.encode()))
 
     def _format(self, fn):
         need = ctypes.c_size_t(0)
@@ -483,6 +499,13 @@ class Context:
                                          ply_path.encode() if ply_path else None, ctypes.byref(rep)))
         return rep
 
+    def export_indexed(self, scene_dir, grid_level=0, ply_path=None, normals=False):
+        """dcsg_export_indexed: the export pipeline writing the indexed PLY (adaptive meshes welded before the projection)."""
+        rep = ExportReport()
+        self._check(self.lib.dcsg_export_indexed(self.h, scene_dir.encode(), grid_level, PLY_NORMALS if normals else 0,
+                                                 ply_path.encode(), ctypes.byref(rep)))
+        return rep
+
 
 def comm_unique_id():
     """dcsg_comm_unique_id: 128 bytes rank 0 creates and hands to the other ranks (any side channel)."""
@@ -541,6 +564,13 @@ class Comm:
         self.ctx._check(self.ctx.lib.dcsg_export_sharded(self.ctx.h, self.h, scene_dir.encode(), grid_level,
                                                          stl_path.encode() if stl_path else None, ply_path.encode() if ply_path else None,
                                                          ctypes.byref(rep)))
+        return rep
+
+    def export_indexed(self, scene_dir, grid_level, ply_path, normals=False):
+        """dcsg_export_sharded_indexed: the indexed PLY over all ranks; uniform lattice (grid_level > 0) only."""
+        rep = ExportReport()
+        self.ctx._check(self.ctx.lib.dcsg_export_sharded_indexed(self.ctx.h, self.h, scene_dir.encode(), grid_level,
+                                                                 PLY_NORMALS if normals else 0, ply_path.encode(), ctypes.byref(rep)))
         return rep
 
 

@@ -169,12 +169,14 @@ static int host_expand_permille(const dcsg_ctx* ctx) {
     const char* e = getenv("DCSG_HOST_EXPAND_PERMILLE");        // read per call: a handful of calls per export
     return e ? atoi(e) : (ctx->node_ranks > 1 ? 0 : 600);
 }
-static int host_threads(const dcsg_ctx* ctx) {
+}  // extern "C"
+int dcsg_host::host_threads(const dcsg_ctx* ctx) {
     const char* e = getenv("DCSG_HOST_THREADS");
     const int cores = (int)std::max(4u, std::thread::hardware_concurrency());
     const int n = e ? atoi(e) : std::min(16, std::max(2, cores / std::max(1, ctx->node_ranks)));
     return std::max(1, std::min(64, n));
 }
+extern "C" {
 
 struct FileTargets { FileSink* sink; int fdPly, fdStl; uint64_t totalTriangles; size_t plyHeader; };
 

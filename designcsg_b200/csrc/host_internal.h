@@ -192,7 +192,8 @@ struct dcsg_ctx {
 
     // workspace
     dcsg_host::DevBuf pts, vals, axes, sign, leaf, cfail, coarse, levels, alive, vinfo, tiles, small, lattice_values, fmt,
-           adapt_emit, adapt_snap, search_bits, project_cursor, project_list, lists, masks, soup;
+           adapt_emit, adapt_snap, search_bits, project_cursor, project_list, lists, masks, soup,
+           weld;                    // dcsg_mesh_weld: sort / scan scratch, then the compacted vertices and normals
     dcsg_host::HostBuf pinned, pinned_small, pinned_soup;
     // sparse extraction: `leaf` (as leafAlive) and `alive` are all-zero between extractions -- every sparse
     // extraction zeroes the words it wrote (dcsg_launch_cleanup); anything else that writes them clears this flag
@@ -438,6 +439,8 @@ struct MeshStorage {        // owned by a dcsg_mesh through `reserved`
 
 // host_files.cu
 std::string ply_header(uint64_t tris);
+// FileSink threads for the file pipelines (DCSG_HOST_THREADS)
+int host_threads(const dcsg_ctx* ctx);
 // exportConfig.txt, positional (reference DesignCSG.cpp:827-835), without exceptions; fills the octree levels, the threshold,
 // the projection steps and the search diameter
 int parse_export_config(dcsg_ctx* ctx, dcsg_extract_cfg& cfg, float& search_diameter);

@@ -108,6 +108,30 @@ void dcsg_launch_format_ply_faces(uint64_t firstTriangle, uint64_t numTriangles,
 void dcsg_launch_expand_soup(const float* vertices, const uint32_t* triangles, uint64_t numTriangles,
                              float* out, cudaStream_t s);
 
+// rows of the indexed binary PLY (dcsg_write_ply_indexed): face rows = the byte 3 and the triangle's vertex ids + base as
+// little-endian uint32 (13 B); vertex rows with normals = x y z nx ny nz as float (24 B).  Without normals the vertex rows
+// are the bytes of the vertex array itself.
+void dcsg_launch_format_ply_indexed_faces(const uint32_t* triangles, uint64_t numTriangles, uint32_t base,
+                                          uint8_t* out /* 13 B per triangle */, cudaStream_t s);
+void dcsg_launch_format_ply_indexed_vertices(const float* vertices, const float* normals, uint64_t numVertices,
+                                             float* out /* 6 floats per vertex */, cudaStream_t s);
+
+// Weld: vertices whose three position words are bit-identical become one vertex, numbered in the order of the smallest input
+// index among them.  The unique vertices (and normals, if any) are compacted into outVertices / outNormals, the triangles are
+// renumbered in place, and *unique (device) receives the new vertex count.  Deterministic; n < 2^32.
+struct dcsg_weld_params {
+    const float* vertices;
+    const float* normals;           // or NULL
+    uint32_t* triangles;
+    uint64_t numVertices, numTriangles;
+    void* scratch;                  // dcsg_weld_scratch_bytes(numVertices) bytes of device memory
+    float* outVertices;             // 3 floats per input vertex
+    float* outNormals;              // idem, when normals != NULL
+    uint32_t* unique;
+};
+size_t dcsg_weld_scratch_bytes(uint64_t numVertices);
+cudaError_t dcsg_launch_weld(const dcsg_weld_params& p, cudaStream_t s);
+
 // ---- adaptive octree mode (mesher_kernels.cu "adaptive") ----------------------------------------------
 struct dcsg_adapt_emit_params {
     dcsg_grid g;                    // the slab of sample planes the sign bitmap covers (z0 = its first plane)

@@ -240,6 +240,26 @@ int  dcsg_set_progress_callback(dcsg_ctx* ctx, dcsg_progress_fn fn, void* user);
 /* Number of CUDA kernels this library has launched in this process (measurement support). */
 unsigned long long dcsg_launch_count(void);
 
+/* ---- indexed binary PLY (no reference counterpart: the reference writes triangle soup only, utils.hpp:41-154) ----------------
+ * An opt-in format beside the reference's files, which stay as they are.  Binary little-endian, header:
+ *   ply / format binary_little_endian 1.0 / comment DesignCSG export, indexed: vertices shared between faces /
+ *   element vertex V / property float x, y, z [/ property float nx, ny, nz  with DCSG_PLY_NORMALS] /
+ *   element face T / property list uchar uint vertex_indices / end_header
+ * then V vertex rows (12 B, 24 B with normals) and T face rows (the byte 3, three uint32 vertex ids: 13 B).  Face i is triangle i
+ * of the reference's files, same corner order, degenerate faces kept: expanding the file, double(vertex[face]), gives the
+ * vertex rows of the soup PLY byte for byte.  V < 2^32. */
+#define DCSG_PLY_NORMALS 1
+
+/* Weld (no reference counterpart): vertices whose positions are bit-identical (all three float words equal) become one, numbered
+ * in the order of the smallest input index among them; triangles are renumbered, normals follow their vertices, num_vertices
+ * shrinks, host copies (copy_to_host) are refreshed.  Deterministic.  Applies to the positions the mesh holds at the call.
+ * A lattice mesh (vertex keys) is returned unchanged: it holds every position once already.  A slab of a sharded adaptive
+ * extraction is refused (DCSG_ERR_UNSUPPORTED).  A welded adaptive mesh is no longer accepted by the soup file pipeline
+ * (dcsg_project_and_*); dcsg_project, dcsg_mesh_soup and the soup writers work on it and give the same bytes as before. */
+int  dcsg_mesh_weld(dcsg_ctx* ctx, dcsg_mesh* mesh);
+/* The indexed PLY of a mesh as it is (no projection); flags & DCSG_PLY_NORMALS needs d_normals.  No reference counterpart. */
+int  dcsg_write_ply_indexed(dcsg_ctx* ctx, const dcsg_mesh* mesh, int flags, const char* path);
+
 typedef struct dcsg_export_report {
     float    box[6];
     uint64_t num_vertices, num_triangles, num_cells;
@@ -251,6 +271,14 @@ typedef struct dcsg_export_report {
  * NULL. */
 int  dcsg_export(dcsg_ctx* ctx, const char* scene_dir, int grid_level_override, const char* stl_path,
                  const char* ply_path, dcsg_export_report* report);
+
+/* dcsg_export's pipeline writing the indexed PLY instead of the soup files (no reference counterpart): bbox -> extract (the
+ * reference's retopologize included) -> adaptive levels: weld BEFORE the projection (equal starting positions project to equal
+ * positions and normals, so each is projected once) -> projection in chunks of vertices pipelined with the copies and the
+ * writes; the face rows are formatted and copied while the projection runs.  Same progress states as dcsg_export; while the
+ * file is written, done / total of DCSG_PROGRESS_WRITING_PLY count vertex rows.  report->num_vertices = the file's vertices. */
+int  dcsg_export_indexed(dcsg_ctx* ctx, const char* scene_dir, int grid_level_override, int flags, const char* ply_path,
+                         dcsg_export_report* report);
 
 /* ---- multi-GPU export: one process per GPU, one node (no reference counterpart: the reference's export runs on one OpenCL
  * device, DesignCSG.cpp:638-790).  The lattice is cut into z-slabs, one per rank.  NCCL carries the small collectives (the
@@ -299,6 +327,14 @@ int  dcsg_extract_sharded(dcsg_ctx* ctx, dcsg_comm* comm, const dcsg_extract_cfg
  * canonical order is (level, node), and every rank writes one byte range per octree level.  Collective. */
 int  dcsg_export_sharded(dcsg_ctx* ctx, dcsg_comm* comm, const char* scene_dir, int grid_level_override, const char* stl_path,
                          const char* ply_path, dcsg_export_report* report);
+
+/* dcsg_export_indexed over all ranks, uniform lattice only (grid_level_override > 0; no reference counterpart).  Rank r
+ * projects and writes only the vertices its slab owns, at header + row bytes * first_vertex, and its face rows with ids +
+ * first_vertex at header + row bytes * total_vertices + 13 * first_triangle; rank 0 creates the file.  Same file as
+ * dcsg_export_indexed on one GPU, byte for byte.  Adaptive levels return DCSG_ERR_UNSUPPORTED on every rank before the first
+ * collective (the weld spans slabs).  Collective. */
+int  dcsg_export_sharded_indexed(dcsg_ctx* ctx, dcsg_comm* comm, const char* scene_dir, int grid_level_override, int flags,
+                                 const char* ply_path, dcsg_export_report* report);
 
 /* Multi-GPU: z-slab boundaries (cell layers, multiples of `granularity`) that give `world` ranks about the same
  * amount of surface, estimated from the per-z sign-change counts of the last dcsg_bbox search on this context.
