@@ -1,13 +1,11 @@
 // host_indexed.cu -- the indexed binary PLY (vertices shared between faces, optional normals): the weld of adaptive meshes,
-// the projection / format / copy / write pipeline of that file, and the single- and multi-GPU exports that write it.
+// and the projection / format / copy / write pipeline of that file (the exports that write it: host_files.cu).
 // An opt-in format beyond the reference's soup files (host_files.cu), which stay the default and unchanged.
 #include "host_internal.h"
 
 using namespace dcsg_host;
 
-namespace {
-
-std::string indexed_ply_header(uint64_t vertices, uint64_t triangles, bool normals) {
+std::string dcsg_host::indexed_ply_header(uint64_t vertices, uint64_t triangles, bool normals) {
     return format("ply\nformat binary_little_endian 1.0\n"
                   "comment DesignCSG export, indexed: vertices shared between faces\n"
                   "element vertex %llu\nproperty float x\nproperty float y\nproperty float z\n%s"
@@ -16,7 +14,7 @@ std::string indexed_ply_header(uint64_t vertices, uint64_t triangles, bool norma
                   (unsigned long long)triangles);
 }
 
-int weld_locked(dcsg_ctx* ctx, dcsg_mesh* mesh) {
+int dcsg_host::weld_locked(dcsg_ctx* ctx, dcsg_mesh* mesh) {
     CUDA_TRY(ctx, cudaSetDevice(ctx->device));
     MeshStorage* st = (MeshStorage*)mesh->reserved;
     if (mesh->d_vertex_keys) return DCSG_OK;        // a lattice mesh holds every position once already (one per lattice edge)
@@ -64,19 +62,9 @@ int weld_locked(dcsg_ctx* ctx, dcsg_mesh* mesh) {
     return DCSG_OK;
 }
 
-// Where a mesh's rows go in the indexed file: vertex rows [0, vertices) of the mesh at vertexOffset, all its face rows (ids +
-// base) at faceOffset.
-struct IndexedTarget {
-    int fd;
-    uint64_t vertexOffset, faceOffset;
-    uint32_t base;
-    uint64_t vertices;
-};
-
-// gd_steps >= 0: project the vertices (and compute the normals) chunk by chunk, pipelined with the copies and the writes;
-// gd_steps < 0: the mesh is final (its d_normals are written).  The face rows do not depend on the projection: they are
-// formatted and copied on the copy stream while the first chunks are projected.
-int indexed_pipeline_locked(dcsg_ctx* ctx, dcsg_mesh* mesh, int gd_steps, bool normals, const IndexedTarget& t) {
+// The face rows do not depend on the projection: they are formatted and copied on the copy stream while the first chunks
+// are projected.
+int dcsg_host::indexed_pipeline_locked(dcsg_ctx* ctx, dcsg_mesh* mesh, int gd_steps, bool normals, const IndexedTarget& t) {
     CUDA_TRY(ctx, cudaSetDevice(ctx->device));
     MeshStorage* st = (MeshStorage*)mesh->reserved;
     const bool project = gd_steps >= 0;
@@ -157,31 +145,6 @@ int indexed_pipeline_locked(dcsg_ctx* ctx, dcsg_mesh* mesh, int gd_steps, bool n
     return ok ? DCSG_OK : fail(ctx, DCSG_ERR_IO, "short write");
 }
 
-// creates the file at its final size with the header in place; returns the descriptor or -1
-int create_indexed_file(const char* path, const std::string& header, uint64_t size) {
-    const int fd = open(path, O_RDWR | O_CREAT | O_TRUNC, 0644);
-    if (fd < 0) return -1;
-    if (ftruncate(fd, (off_t)size) != 0 || pwrite(fd, header.data(), header.size(), 0) != (ssize_t)header.size()) {
-        close(fd);
-        return -1;
-    }
-    return fd;
-}
-
-// exportConfig.txt with the export's fixed choices (retopologize, the level override) -- what dcsg_export runs
-int export_config(dcsg_ctx* ctx, const char* scene_dir, int grid_level_override, dcsg_extract_cfg& cfg, float& search) {
-    int rc = dcsg_build(ctx, scene_dir, nullptr, 0);
-    if (rc != DCSG_OK) return rc;
-    rc = parse_export_config(ctx, cfg, search);
-    if (rc != DCSG_OK) return rc;
-    cfg.retopologize = 1;
-    if (grid_level_override > 0) cfg.min_level = cfg.max_level = cfg.grid_level = grid_level_override;
-    cfg.defer_projection = 1;
-    return DCSG_OK;
-}
-
-}  // namespace
-
 extern "C" {
 
 int dcsg_mesh_weld(dcsg_ctx* ctx, dcsg_mesh* mesh) {
@@ -199,135 +162,10 @@ int dcsg_write_ply_indexed(dcsg_ctx* ctx, const dcsg_mesh* mesh_in, int flags, c
     if (mesh.num_vertices > 0xffffffffull) return fail(ctx, DCSG_ERR_INVALID, "more than 2^32 vertices");
     const uint64_t V = mesh.num_vertices, T = mesh.num_triangles, row = normals ? 24 : 12;
     const std::string header = indexed_ply_header(V, T, normals);
-    const int fd = create_indexed_file(path, header, header.size() + row * V + 13 * T);
+    const int fd = create_sized_file(path, header, header.size() + row * V + 13 * T);
     if (fd < 0) return fail(ctx, DCSG_ERR_IO, std::string("cannot create ") + path);
     const int rc = indexed_pipeline_locked(ctx, &mesh, -1, normals, IndexedTarget{fd, header.size(), header.size() + row * V, 0u, V});
     close(fd);
-    return rc;
-}
-
-int dcsg_export_indexed(dcsg_ctx* ctx, const char* scene_dir, int grid_level_override, int flags, const char* ply_path,
-                        dcsg_export_report* report) {
-    if (!ctx || !scene_dir || !ply_path || (flags & ~DCSG_PLY_NORMALS)) return DCSG_ERR_INVALID;
-    const double t0 = now_ms();
-    dcsg_extract_cfg cfg;
-    float search = 0.0f;
-    int rc = export_config(ctx, scene_dir, grid_level_override, cfg, search);
-    if (rc != DCSG_OK) return rc;
-    const bool normals = (flags & DCSG_PLY_NORMALS) != 0;
-    dcsg_export_report rep;
-    memset(&rep, 0, sizeof(rep));
-    double t = now_ms();
-    report_progress(ctx, DCSG_PROGRESS_ESTIMATING_BOUNDING_BOX, 0, 0);
-    rc = dcsg_bbox(ctx, search, cfg.box);
-    if (rc != DCSG_OK) return rc;
-    rep.bbox_ms = (float)(now_ms() - t);
-    memcpy(rep.box, cfg.box, sizeof(rep.box));
-    dcsg_mesh mesh;
-    memset(&mesh, 0, sizeof(mesh));
-    report_progress(ctx, DCSG_PROGRESS_PERFORMING_CMS, 0, 0);
-    rc = dcsg_extract(ctx, &cfg, &mesh);
-    if (rc != DCSG_OK) { dcsg_mesh_free(ctx, &mesh); return rc; }
-    report_progress(ctx, DCSG_PROGRESS_RETOPOLOGIZING, 0, 0);
-    memcpy(rep.extract_ms, mesh.stage_ms, sizeof(rep.extract_ms));
-    t = now_ms();
-    {
-        std::lock_guard<std::mutex> g(ctx->lock);
-        // adaptive walk: equal pre-projection positions project to equal positions and normals, so welding first projects each
-        // position once and gives the same file as welding after the projection (a lattice mesh is returned unchanged)
-        rc = weld_locked(ctx, &mesh);
-        if (rc == DCSG_OK && mesh.num_vertices > 0xffffffffull) rc = fail(ctx, DCSG_ERR_INVALID, "more than 2^32 vertices");
-        report_progress(ctx, DCSG_PROGRESS_GRADIENT_DESCENT, 0, (uint64_t)std::max(cfg.gd_steps, 0));
-        if (rc == DCSG_OK) {
-            const uint64_t V = mesh.num_vertices, T = mesh.num_triangles, row = normals ? 24 : 12;
-            const std::string header = indexed_ply_header(V, T, normals);
-            const int fd = create_indexed_file(ply_path, header, header.size() + row * V + 13 * T);
-            if (fd < 0) rc = fail(ctx, DCSG_ERR_IO, std::string("cannot create ") + ply_path);
-            else {
-                rc = indexed_pipeline_locked(ctx, &mesh, std::max(cfg.gd_steps, 0), normals,
-                                             IndexedTarget{fd, header.size(), header.size() + row * V, 0u, V});
-                close(fd);
-            }
-        }
-    }
-    rep.write_ms = (float)(now_ms() - t);
-    rep.num_vertices = mesh.num_vertices;
-    rep.num_triangles = mesh.num_triangles;
-    rep.num_cells = mesh.num_cells;
-    if (rc == DCSG_OK) report_progress(ctx, DCSG_PROGRESS_COMPLETE, mesh.num_triangles, mesh.num_triangles);
-    dcsg_mesh_free(ctx, &mesh);
-    rep.total_ms = (float)(now_ms() - t0);
-    if (report) *report = rep;
-    return rc;
-}
-
-int dcsg_export_sharded_indexed(dcsg_ctx* ctx, dcsg_comm* c, const char* scene_dir, int grid_level_override, int flags,
-                                const char* ply_path, dcsg_export_report* report) {
-    if (!ctx || !c || !scene_dir || !ply_path || (flags & ~DCSG_PLY_NORMALS)) return DCSG_ERR_INVALID;
-    const double t0 = now_ms();
-    dcsg_extract_cfg cfg;
-    float search = 0.0f;
-    int rc = export_config(ctx, scene_dir, grid_level_override, cfg, search);
-    if (rc != DCSG_OK) return rc;
-    // decided from exportConfig.txt alone, the same on every rank, before the first collective
-    if (!(cfg.min_level >= cfg.grid_level && cfg.max_level == cfg.grid_level))
-        return fail(ctx, DCSG_ERR_UNSUPPORTED, "the sharded indexed export needs a uniform lattice (grid_level_override > 0): the weld of an adaptive mesh spans slabs");
-    const bool normals = (flags & DCSG_PLY_NORMALS) != 0;
-    dcsg_export_report rep;
-    memset(&rep, 0, sizeof(rep));
-    double t = now_ms();
-    report_progress(ctx, DCSG_PROGRESS_ESTIMATING_BOUNDING_BOX, 0, 0);
-    rc = dcsg_bbox_sharded(ctx, c, search, cfg.box);
-    if (rc != DCSG_OK) return rc;
-    rep.bbox_ms = (float)(now_ms() - t);
-    memcpy(rep.box, cfg.box, sizeof(rep.box));
-    dcsg_mesh mesh;
-    memset(&mesh, 0, sizeof(mesh));
-    dcsg_shard_info info;
-    report_progress(ctx, DCSG_PROGRESS_PERFORMING_CMS, 0, 0);
-    rc = dcsg_extract_sharded(ctx, c, &cfg, -1, &mesh, nullptr, &info);
-    if (rc != DCSG_OK) { dcsg_mesh_free(ctx, &mesh); return rc; }
-    memcpy(rep.extract_ms, mesh.stage_ms, sizeof(rep.extract_ms));
-    rep.num_vertices = info.total_vertices;
-    rep.num_triangles = info.total_triangles;
-    rep.num_cells = info.total_cells;
-    if (info.total_vertices > 0xffffffffull) {         // the same counts on every rank: all return here
-        dcsg_mesh_free(ctx, &mesh);
-        return fail(ctx, DCSG_ERR_INVALID, "more than 2^32 vertices");
-    }
-    report_progress(ctx, DCSG_PROGRESS_RETOPOLOGIZING, 0, 0);
-    report_progress(ctx, DCSG_PROGRESS_GRADIENT_DESCENT, 0, (uint64_t)std::max(cfg.gd_steps, 0));
-    t = now_ms();
-    const uint64_t row = normals ? 24 : 12;
-    const std::string header = indexed_ply_header(info.total_vertices, info.total_triangles, normals);
-    // rank 0 creates the file at its final size and writes the header; then every rank writes its own vertex rows (the slab's
-    // owned vertices: the ranks' owned vertices in rank order are the whole mesh's) and its face rows (ids + first_vertex)
-    if (dcsg_comm_rank(c) == 0) {
-        const int fd = create_indexed_file(ply_path, header, header.size() + row * info.total_vertices + 13 * info.total_triangles);
-        if (fd < 0) rc = fail(ctx, DCSG_ERR_IO, std::string("cannot create ") + ply_path);
-        else close(fd);
-    }
-    int brc = dcsg_comm_barrier(c);
-    if (rc == DCSG_OK) rc = brc;
-    if (rc == DCSG_OK) {
-        const int fd = open(ply_path, O_WRONLY);
-        if (fd < 0) rc = fail(ctx, DCSG_ERR_IO, std::string("cannot open ") + ply_path);
-        else {
-            std::lock_guard<std::mutex> g(ctx->lock);
-            rc = indexed_pipeline_locked(ctx, &mesh, std::max(cfg.gd_steps, 0), normals,
-                                         IndexedTarget{fd, header.size() + row * info.first_vertex,
-                                                       header.size() + row * info.total_vertices + 13 * info.first_triangle,
-                                                       (uint32_t)info.first_vertex, mesh.owned_vertices});
-            close(fd);
-        }
-    }
-    brc = dcsg_comm_barrier(c);
-    if (rc == DCSG_OK) rc = brc;
-    rep.write_ms = (float)(now_ms() - t);
-    if (rc == DCSG_OK) report_progress(ctx, DCSG_PROGRESS_COMPLETE, info.total_triangles, info.total_triangles);
-    dcsg_mesh_free(ctx, &mesh);
-    rep.total_ms = (float)(now_ms() - t0);
-    if (report) *report = rep;
     return rc;
 }
 
