@@ -5,6 +5,8 @@
     python -m designcsg_b200 export  SCENE_DIR|DESIGN.py --ply-indexed P [--normals] [--level L]
                                                                        indexed binary PLY (shared float vertices, optional
                                                                        normals; not the reference's format)
+    ... export ... --outward                                           every triangle wound to face out of the solid (any of
+                                                                       the files above; not the reference's bytes)
     torchrun --nproc-per-node G -m designcsg_b200 export ...          z-slab sharded over G GPUs (dcsg_export_sharded; the
                                                                        same export from a C host: tools/dcsg_mgpu.c)
 """
@@ -77,7 +79,7 @@ def cmd_export(args):
     report = {"scene": scene, "octree_levels": [lo, hi, level], "gd_steps": steps, "gpus": world, "build_s": t_build}
     if world == 1 and args.ply_indexed:
         t1 = time.perf_counter()
-        rep = ctx.export_indexed(scene, args.level, args.ply_indexed, normals=args.normals)
+        rep = ctx.export_indexed(scene, args.level, args.ply_indexed, normals=args.normals, outward=args.outward)
         report.update(triangles=int(rep.num_triangles), vertices=int(rep.num_vertices), box=[float(v) for v in rep.box],
                       export_s=time.perf_counter() - t1, project_and_write_ms=float(rep.write_ms))
     elif world == 1:
@@ -88,6 +90,8 @@ def cmd_export(args):
                            complex_threshold=threshold, retopologize=not args.no_retopologize, defer_projection=pipelined)
         report.update(triangles=mesh.num_triangles, vertices=mesh.num_vertices, stage_ms=mesh.stage_ms)
         t1 = time.perf_counter()
+        if args.outward:
+            mesh.orient()
         if pipelined:
             mesh.project_and_write_files(steps, args.stl, args.ply)
         else:
@@ -111,9 +115,9 @@ def cmd_export(args):
         comm = D.create_comm(ctx)       # from here on everything collective happens inside libdcsg
         t1 = time.perf_counter()
         if args.ply_indexed:
-            rep = comm.export_indexed(scene, args.level, args.ply_indexed, normals=args.normals)
+            rep = comm.export_indexed(scene, args.level, args.ply_indexed, normals=args.normals, outward=args.outward)
         else:
-            rep = comm.export(scene, args.level, args.stl, args.ply)
+            rep = comm.export(scene, args.level, args.stl, args.ply, outward=args.outward)
         report.update(triangles=int(rep.num_triangles), vertices=int(rep.num_vertices), box=[float(v) for v in rep.box],
                       export_s=time.perf_counter() - t1, search_ms=float(rep.bbox_ms), project_and_write_ms=float(rep.write_ms))
         comm.close()
@@ -141,6 +145,8 @@ def main():
     e.add_argument("--ply-indexed", help="write an indexed binary PLY instead (shared float vertices; with --normals the "
                    "projection's normals too) -- a format beyond the reference's")
     e.add_argument("--normals", action="store_true")
+    e.add_argument("--outward", action="store_true", help="wind every triangle to face out of the solid (dcsg_mesh_orient) in "
+                   "whichever files are written; the files are then not the reference's bytes, whose winding is mixed")
     e.set_defaults(fn=cmd_export)
     args = ap.parse_args()
     args.fn(args)

@@ -66,6 +66,7 @@ PROGRESS_STATES = ("IDLE", "ESTIMATING_BOUNDING_BOX", "PERFORMING_CMS", "RETOPOL
 PROGRESS_FN = ctypes.CFUNCTYPE(None, ctypes.c_void_p, ctypes.c_int, ctypes.c_uint64, ctypes.c_uint64)
 
 PLY_NORMALS = 1                                                 # dcsg.h DCSG_PLY_NORMALS
+EXPORT_OUTWARD = 1                                              # dcsg.h DCSG_EXPORT_OUTWARD
 
 _lib = None
 
@@ -140,6 +141,8 @@ def load_library():
     lib.dcsg_write_ply_indexed.argtypes = [vp, ctypes.POINTER(MeshStruct), ci, cp]
     lib.dcsg_export_indexed.argtypes = [vp, cp, ci, ci, cp, ctypes.POINTER(ExportReport)]
     lib.dcsg_export_sharded_indexed.argtypes = [vp, vp, cp, ci, ci, cp, ctypes.POINTER(ExportReport)]
+    lib.dcsg_mesh_orient.argtypes = [vp, ctypes.POINTER(MeshStruct)]
+    lib.dcsg_set_export_flags.argtypes = [vp, ci]
     _lib = lib
     return lib
 
@@ -302,6 +305,12 @@ class Mesh:
         A lattice mesh comes back unchanged.  The host arrays are refreshed when the mesh was copied to the host."""
         self._ctx._check(self._ctx.lib.dcsg_mesh_weld(self._ctx.h, ctypes.byref(self.c)))
 
+    def orient(self):
+        """dcsg_mesh_orient: swap corners 1 and 2 of the inward-facing triangles so that every triangle faces out of the solid.
+        Vertices, cells and triangle order stay; the host arrays are refreshed when the mesh was copied to the host; a second
+        call changes nothing.  The STL writers then list the corners A, C, B (the files are no longer the reference's bytes)."""
+        self._ctx._check(self._ctx.lib.dcsg_mesh_orient(self._ctx.h, ctypes.byref(self.c)))
+
     def write_ply_indexed(self, path, normals=False):
         """dcsg_write_ply_indexed: binary PLY with shared float vertices (and the mesh's normals) -- not the reference's format."""
         self._ctx._check(self._ctx.lib.dcsg_write_ply_indexed(self._ctx.h, ctypes.byref(self.c), PLY_NORMALS if normals else 0,
@@ -375,6 +384,7 @@ class Context:
             raise DcsgError(rc, "dcsg_create(%d) failed: no usable CUDA device (the export path has no CPU fallback)" % device)
         self.device = device
         self.build_log = ""
+        self._export_flags = 0
 
     def _check(self, rc):
         if rc != 0:
@@ -493,17 +503,37 @@ class Context:
         self._check(self.lib.dcsg_fp32_peak(self.h, mode, ctypes.byref(v)))
         return v.value
 
-    def export(self, scene_dir, grid_level=0, stl_path=None, ply_path=None):
+    def set_export_flags(self, flags):
+        """dcsg_set_export_flags: options of the dcsg_export* calls on this context (EXPORT_OUTWARD)."""
+        self._check(self.lib.dcsg_set_export_flags(self.h, flags))
+        self._export_flags = flags
+
+    def _with_export_flags(self, outward, call):
+        """Run call() with DCSG_EXPORT_OUTWARD set or cleared as asked; the context's flags are restored afterwards."""
+        before = self._export_flags
+        wanted = (before | EXPORT_OUTWARD) if outward else (before & ~EXPORT_OUTWARD)
+        if wanted == before:
+            return call()
+        self.set_export_flags(wanted)
+        try:
+            return call()
+        finally:
+            self.set_export_flags(before)
+
+    def export(self, scene_dir, grid_level=0, stl_path=None, ply_path=None, outward=False):
+        """dcsg_export; outward=True orients the mesh before the files are written (not the reference's bytes then)."""
         rep = ExportReport()
-        self._check(self.lib.dcsg_export(self.h, scene_dir.encode(), grid_level, stl_path.encode() if stl_path else None,
-                                         ply_path.encode() if ply_path else None, ctypes.byref(rep)))
+        self._with_export_flags(outward, lambda: self._check(self.lib.dcsg_export(
+            self.h, scene_dir.encode(), grid_level, stl_path.encode() if stl_path else None, ply_path.encode() if ply_path else None,
+            ctypes.byref(rep))))
         return rep
 
-    def export_indexed(self, scene_dir, grid_level=0, ply_path=None, normals=False):
-        """dcsg_export_indexed: the export pipeline writing the indexed PLY (adaptive meshes welded before the projection)."""
+    def export_indexed(self, scene_dir, grid_level=0, ply_path=None, normals=False, outward=False):
+        """dcsg_export_indexed: the export pipeline writing the indexed PLY (adaptive meshes welded before the projection);
+        outward=True orients the mesh first."""
         rep = ExportReport()
-        self._check(self.lib.dcsg_export_indexed(self.h, scene_dir.encode(), grid_level, PLY_NORMALS if normals else 0,
-                                                 ply_path.encode(), ctypes.byref(rep)))
+        self._with_export_flags(outward, lambda: self._check(self.lib.dcsg_export_indexed(
+            self.h, scene_dir.encode(), grid_level, PLY_NORMALS if normals else 0, ply_path.encode(), ctypes.byref(rep))))
         return rep
 
 
@@ -559,18 +589,19 @@ class Comm:
         whole._borrowed = True
         return mesh, whole, info
 
-    def export(self, scene_dir, grid_level=0, stl_path=None, ply_path=None):
+    def export(self, scene_dir, grid_level=0, stl_path=None, ply_path=None, outward=False):
+        """dcsg_export_sharded; outward=True orients every rank's slab before the files are written."""
         rep = ExportReport()
-        self.ctx._check(self.ctx.lib.dcsg_export_sharded(self.ctx.h, self.h, scene_dir.encode(), grid_level,
-                                                         stl_path.encode() if stl_path else None, ply_path.encode() if ply_path else None,
-                                                         ctypes.byref(rep)))
+        self.ctx._with_export_flags(outward, lambda: self.ctx._check(self.ctx.lib.dcsg_export_sharded(
+            self.ctx.h, self.h, scene_dir.encode(), grid_level, stl_path.encode() if stl_path else None,
+            ply_path.encode() if ply_path else None, ctypes.byref(rep))))
         return rep
 
-    def export_indexed(self, scene_dir, grid_level, ply_path, normals=False):
+    def export_indexed(self, scene_dir, grid_level, ply_path, normals=False, outward=False):
         """dcsg_export_sharded_indexed: the indexed PLY over all ranks; uniform lattice (grid_level > 0) only."""
         rep = ExportReport()
-        self.ctx._check(self.ctx.lib.dcsg_export_sharded_indexed(self.ctx.h, self.h, scene_dir.encode(), grid_level,
-                                                                 PLY_NORMALS if normals else 0, ply_path.encode(), ctypes.byref(rep)))
+        self.ctx._with_export_flags(outward, lambda: self.ctx._check(self.ctx.lib.dcsg_export_sharded_indexed(
+            self.ctx.h, self.h, scene_dir.encode(), grid_level, PLY_NORMALS if normals else 0, ply_path.encode(), ctypes.byref(rep))))
         return rep
 
 

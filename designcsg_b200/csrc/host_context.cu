@@ -39,8 +39,10 @@ int dcsg_create(int device, dcsg_ctx** out) {
     cudaEventCreateWithFlags(&ctx->aux_done, cudaEventDisableTiming);
     cudaMalloc((void**)&ctx->d_tri_count, 256);
     cudaMalloc((void**)&ctx->d_tri_table, 256 * 16);
+    cudaMalloc((void**)&ctx->d_tri_flip, 256);
     cudaMemcpy(ctx->d_tri_count, kDcsgTriCount, 256, cudaMemcpyHostToDevice);
     cudaMemcpy(ctx->d_tri_table, kDcsgTriTable, 256 * 16, cudaMemcpyHostToDevice);
+    cudaMemcpy(ctx->d_tri_flip, kDcsgTriFlip, 256, cudaMemcpyHostToDevice);
     if (cudaGetLastError() != cudaSuccess) { delete ctx; return DCSG_ERR_CUDA; }
     *out = ctx;
     return DCSG_OK;
@@ -51,7 +53,7 @@ void dcsg_destroy(dcsg_ctx* ctx) {
     cudaSetDevice(ctx->device);
     cudaStreamSynchronize(ctx->stream);
     for (DevBuf* b : {&ctx->pts, &ctx->vals, &ctx->axes, &ctx->sign, &ctx->leaf, &ctx->cfail, &ctx->coarse, &ctx->levels, &ctx->alive, &ctx->vinfo,
-                      &ctx->tiles, &ctx->small, &ctx->lattice_values, &ctx->fmt, &ctx->adapt_emit, &ctx->adapt_snap, &ctx->search_bits, &ctx->project_cursor, &ctx->lists, &ctx->masks, &ctx->soup, &ctx->project_list, &ctx->weld})
+                      &ctx->tiles, &ctx->small, &ctx->lattice_values, &ctx->fmt, &ctx->adapt_emit, &ctx->adapt_snap, &ctx->search_bits, &ctx->project_cursor, &ctx->lists, &ctx->masks, &ctx->soup, &ctx->project_list, &ctx->weld, &ctx->orient})
         b->release();
     ctx->pinned.release();
     ctx->pinned_small.release();
@@ -59,6 +61,7 @@ void dcsg_destroy(dcsg_ctx* ctx) {
     if (ctx->lib) cudaLibraryUnload(ctx->lib);
     cudaFree(ctx->d_tri_count);
     cudaFree(ctx->d_tri_table);
+    cudaFree(ctx->d_tri_flip);
     for (auto& ev : ctx->ev) if (ev) cudaEventDestroy(ev);
     if (ctx->own_stream && ctx->stream) cudaStreamDestroy(ctx->stream);
     if (ctx->copy_stream) cudaStreamDestroy(ctx->copy_stream);
@@ -85,6 +88,13 @@ int dcsg_set_progress_callback(dcsg_ctx* ctx, dcsg_progress_fn fn, void* user) {
     std::lock_guard<std::mutex> g(ctx->lock);
     ctx->progress = fn;
     ctx->progress_user = fn ? user : nullptr;
+    return DCSG_OK;
+}
+
+int dcsg_set_export_flags(dcsg_ctx* ctx, int flags) {
+    if (!ctx || (flags & ~DCSG_EXPORT_OUTWARD)) return DCSG_ERR_INVALID;
+    std::lock_guard<std::mutex> g(ctx->lock);
+    ctx->export_flags = flags;
     return DCSG_OK;
 }
 

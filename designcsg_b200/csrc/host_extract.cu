@@ -672,6 +672,8 @@ int dcsg_extract(dcsg_ctx* ctx, const dcsg_extract_cfg* cfg, dcsg_mesh* out) {
     st->planeVertFirst.clear();
     st->levelTriangles.clear();
     st->runs.clear();
+    st->cellUnit = 0;
+    st->oriented = false;
     if (!uniform) {
         ctx->sparse_clean = false;              // the dense lattice pass writes the bitmaps the sparse pass keeps all-zero
         rc = extract_adaptive(ctx, cfg, s, st, nVerts, nTris, nCells, evals);
@@ -852,6 +854,7 @@ int dcsg_extract(dcsg_ctx* ctx, const dcsg_extract_cfg* cfg, dcsg_mesh* out) {
         st->unitTriangles = points >= 2 ? 3 * points - 2 : 1;
         st->unitVertices = points >= 2 ? 3 * points : 3;
     }
+    st->cellUnit = uniform ? 1 : st->unitTriangles;
     out->owned_vertices = nVerts - nHalo;
     out->halo_vertices = nHalo;
     out->h_vertices = out->h_normals = nullptr;
@@ -904,5 +907,50 @@ int dcsg_mesh_soup(dcsg_ctx* ctx, const dcsg_mesh* mesh, float* out_host) {
     return DCSG_OK;
 }
 
+int dcsg_mesh_orient(dcsg_ctx* ctx, dcsg_mesh* mesh) {
+    if (!ctx || !mesh) return DCSG_ERR_INVALID;
+    std::lock_guard<std::mutex> g(ctx->lock);
+    return orient_locked(ctx, mesh);
+}
+
 }  // extern "C"
+
+// The winding of a triangle is a function of its cell's corner mask and its slot in the table row (tools/gen_mc_table.py), so
+// orienting a mesh is one pass over its cells: no geometry, the same on every schedule, slab and octree level.
+int dcsg_host::orient_locked(dcsg_ctx* ctx, dcsg_mesh* mesh) {
+    MeshStorage* st = (MeshStorage*)mesh->reserved;
+    if (!st || !st->cellUnit || (mesh->num_cells && !mesh->d_cell_masks))
+        return fail(ctx, DCSG_ERR_INVALID, "dcsg_mesh_orient needs a mesh from dcsg_extract: its cells' corner masks decide the winding");
+    if (st->oriented) return DCSG_OK;
+    CUDA_TRY(ctx, cudaSetDevice(ctx->device));
+    const uint64_t n = mesh->num_cells;
+    auto align = [](size_t v) { return (v + 255) & ~(size_t)255; };
+    const size_t scratch = align(dcsg_orient_scratch_bytes(n));
+    CUDA_TRY(ctx, ctx->orient.reserve(scratch + 256));
+    uint8_t* w = ctx->orient.as<uint8_t>();
+    dcsg_orient_params p;
+    p.cellMasks = mesh->d_cell_masks;
+    p.numCells = n;
+    p.triCount = ctx->d_tri_count;
+    p.triFlip = ctx->d_tri_flip;
+    p.unit = (uint32_t)st->cellUnit;
+    p.triangles = mesh->d_triangles;
+    p.numTriangles = mesh->num_triangles;
+    p.scratch = w;
+    p.total = reinterpret_cast<uint32_t*>(w + scratch);
+    cudaStream_t s = ctx->stream;
+    CUDA_TRY(ctx, dcsg_launch_orient(p, s));
+    g_launches += 2;                // the count and the swap; cub's scan passes are not counted
+    CUDA_TRY(ctx, ctx->pinned_small.reserve(64));
+    uint32_t* h_total = ctx->pinned_small.as<uint32_t>();
+    CUDA_TRY(ctx, cudaMemcpyAsync(h_total, p.total, 4, cudaMemcpyDeviceToHost, s));
+    if (mesh->h_triangles && mesh->num_triangles)
+        CUDA_TRY(ctx, cudaMemcpyAsync(mesh->h_triangles, mesh->d_triangles, mesh->num_triangles * 12, cudaMemcpyDeviceToHost, s));
+    CUDA_TRY(ctx, cudaStreamSynchronize(s));
+    if (*h_total != mesh->num_triangles)
+        return fail(ctx, DCSG_ERR_INVALID, format("dcsg_mesh_orient: the cells account for %u triangles, the mesh holds %llu", *h_total,
+                                                  (unsigned long long)mesh->num_triangles));
+    st->oriented = true;
+    return DCSG_OK;
+}
 

@@ -73,6 +73,13 @@ int dcsg_host::host_threads(const dcsg_ctx* ctx) {
     return std::max(1, std::min(64, n));
 }
 
+// An outward-wound mesh (dcsg_mesh_orient) lists its STL corners A, C, B: the records store every corner as (x, z, y), and
+// that swap of two axes would turn the winding inside out again.  Meshes the library does not own are written as they are.
+static bool stl_acb(const dcsg_mesh* mesh) {
+    const MeshStorage* st = (const MeshStorage*)mesh->reserved;
+    return st && st->oriented;
+}
+
 extern "C" {
 // Lay the file out in pinned host memory: header bytes by the host, body by the device kernels.
 static int format_locked(dcsg_ctx* ctx, const dcsg_mesh* mesh, bool ply, uint8_t** bytes, size_t* size) {
@@ -91,7 +98,7 @@ static int format_locked(dcsg_ctx* ctx, const dcsg_mesh* mesh, bool ply, uint8_t
             dcsg_launch_format_ply_vertices(mesh->d_vertices, mesh->d_triangles, n, (double*)d, ctx->stream);
             dcsg_launch_format_ply_faces(0, n, d + n * 72, ctx->stream); g_launches += 2;
         } else {
-            dcsg_launch_format_stl(mesh->d_vertices, mesh->d_triangles, n, d, ctx->stream); ++g_launches;
+            dcsg_launch_format_stl(mesh->d_vertices, mesh->d_triangles, n, d, stl_acb(mesh), ctx->stream); ++g_launches;
         }
         CUDA_TRY(ctx, cudaGetLastError());
         CUDA_TRY(ctx, cudaMemcpyAsync(h + header.size(), d, body, cudaMemcpyDeviceToHost, ctx->stream));
@@ -118,7 +125,7 @@ int dcsg_format_segments(dcsg_ctx* ctx, const dcsg_mesh* mesh, uint64_t first_tr
     if (n) {
         dcsg_launch_format_ply_vertices(mesh->d_vertices, mesh->d_triangles, n, (double*)d, ctx->stream);
         dcsg_launch_format_ply_faces(first_triangle, n, d + offFaces, ctx->stream);
-        dcsg_launch_format_stl(mesh->d_vertices, mesh->d_triangles, n, d + offStl, ctx->stream);
+        dcsg_launch_format_stl(mesh->d_vertices, mesh->d_triangles, n, d + offStl, stl_acb(mesh), ctx->stream);
         g_launches += 3;
         CUDA_TRY(ctx, cudaGetLastError());
         CUDA_TRY(ctx, cudaMemcpyAsync(h, d, n * 72, cudaMemcpyDeviceToHost, ctx->stream));
@@ -299,7 +306,7 @@ static int pipeline_locked(dcsg_ctx* ctx, dcsg_mesh* mesh, int gd_steps, uint64_
             const uint64_t split = triEnd - hostTris, m = split - triDone;
             if (m) {
                 dcsg_launch_format_ply_vertices(mesh->d_vertices, mesh->d_triangles + triDone * 3, m, (double*)(d + triDone * 72), cs);
-                dcsg_launch_format_stl(mesh->d_vertices, mesh->d_triangles + triDone * 3, m, d + offStl + triDone * 50, cs);
+                dcsg_launch_format_stl(mesh->d_vertices, mesh->d_triangles + triDone * 3, m, d + offStl + triDone * 50, st->oriented, cs);
                 g_launches += 2;
             }
             if (hostTris) { dcsg_launch_expand_soup(mesh->d_vertices, mesh->d_triangles + split * 3, hostTris, d_soup + soupDone * 9, cs); ++g_launches; }
@@ -331,7 +338,8 @@ static int pipeline_locked(dcsg_ctx* ctx, dcsg_mesh* mesh, int gd_steps, uint64_
             const uint64_t t0 = ranges[c].tri0, split = ranges[c].split;
             const float* soup = h_soup + soupFirst[c] * 9;
             for_each_piece(split, ranges[c].tri1, [&](uint64_t a, uint64_t count, uint64_t global) {
-                pool->submit_expand(soup + (a - split) * 9, count, h + a * 72, h + offStl + a * 50, fdPly, plyRows + 72 * global, fdStl, stlRecords + 50 * global);
+                pool->submit_expand(soup + (a - split) * 9, count, h + a * 72, h + offStl + a * 50, fdPly, plyRows + 72 * global, fdStl,
+                                    stlRecords + 50 * global, st->oriented);
             });
             if (files) {
                 for_each_piece(t0, split, [&](uint64_t a, uint64_t count, uint64_t global) {
@@ -399,7 +407,7 @@ int dcsg_ply_face_rows(uint64_t first_triangle, uint64_t num_triangles, uint8_t*
 
 int dcsg_soup_rows(const float* soup, uint64_t num_triangles, uint8_t* ply_rows, uint8_t* stl_records) {
     if (!soup || !ply_rows || !stl_records || (reinterpret_cast<uintptr_t>(ply_rows) & 7u)) return DCSG_ERR_INVALID;
-    FileSink::expand_rows(soup, num_triangles, ply_rows, stl_records);
+    FileSink::expand_rows(soup, num_triangles, ply_rows, stl_records, false);
     return DCSG_OK;
 }
 
@@ -482,6 +490,11 @@ static int run_export(dcsg_ctx* ctx, dcsg_comm* comm, const char* scene_dir, int
                       dcsg_export_report* report) {
     if (comm && comm_ctx(comm) != ctx) return DCSG_ERR_INVALID;
     const double t0 = now_ms();
+    bool outward;           // dcsg_set_export_flags, read once for the whole export
+    {
+        std::lock_guard<std::mutex> g(ctx->lock);
+        outward = (ctx->export_flags & DCSG_EXPORT_OUTWARD) != 0;
+    }
     dcsg_extract_cfg cfg;
     float search = 0.0f;
     int rc = export_config(ctx, scene_dir, grid_level_override, cfg, search);
@@ -512,8 +525,14 @@ static int run_export(dcsg_ctx* ctx, dcsg_comm* comm, const char* scene_dir, int
     memcpy(rep.extract_ms, mesh.stage_ms, sizeof(rep.extract_ms));
     report_progress(ctx, DCSG_PROGRESS_RETOPOLOGIZING, 0, 0);       // done inside the extraction (identity on a uniform lattice)
     t = now_ms();
+    if (outward) {
+        // right after the extraction, before the weld and the projection: a pure map over (cell, table slot), and every writer
+        // reads the corners through the triangles
+        std::lock_guard<std::mutex> g(ctx->lock);
+        rc = orient_locked(ctx, &mesh);
+    }
     if (!comm) {
-        if (files.indexed) {
+        if (rc == DCSG_OK && files.indexed) {
             // adaptive walk: equal pre-projection positions project to equal positions and normals, so welding first projects
             // each position once and gives the same file as welding after the projection (a lattice mesh is returned unchanged)
             std::lock_guard<std::mutex> g(ctx->lock);

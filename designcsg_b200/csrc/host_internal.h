@@ -172,6 +172,7 @@ struct dcsg_ctx {
     int node_ranks = 1;             // ranks sharing this host (set by dcsg_comm_create): they share its cores and memory bandwidth
     dcsg_progress_fn progress = nullptr;    // optional, see dcsg_set_progress_callback
     void* progress_user = nullptr;
+    int export_flags = 0;           // DCSG_EXPORT_*, see dcsg_set_export_flags
 
     bool built = false;
     uint64_t extract_generation = 0;
@@ -190,11 +191,13 @@ struct dcsg_ctx {
 
     uint8_t* d_tri_count = nullptr;
     int8_t* d_tri_table = nullptr;
+    uint8_t* d_tri_flip = nullptr;          // kDcsgTriFlip: the inward-facing triangles of every table row
 
     // workspace
     dcsg_host::DevBuf pts, vals, axes, sign, leaf, cfail, coarse, levels, alive, vinfo, tiles, small, lattice_values, fmt,
            adapt_emit, adapt_snap, search_bits, project_cursor, project_list, lists, masks, soup,
-           weld;                    // dcsg_mesh_weld: sort / scan scratch, then the compacted vertices and normals
+           weld,                    // dcsg_mesh_weld: sort / scan scratch, then the compacted vertices and normals
+           orient;                  // dcsg_mesh_orient: per-cell counts, their prefix and the scan's scratch
     dcsg_host::HostBuf pinned, pinned_small, pinned_soup;
     // sparse extraction: `leaf` (as leafAlive) and `alive` are all-zero between extractions -- every sparse
     // extraction zeroes the words it wrote (dcsg_launch_cleanup); anything else that writes them clears this flag
@@ -259,6 +262,8 @@ struct LatticeSetup {
 };
 
 // host_extract.cu
+// swaps corners 1 and 2 of the inward-facing triangles (dcsg_mesh_orient); a no-op on an oriented mesh
+int orient_locked(dcsg_ctx* ctx, dcsg_mesh* mesh);
 int setup_lattice(dcsg_ctx* ctx, const float* box, int grid_level, int z0, int z1, LatticeSetup& s, bool check);
 int run_lattice(dcsg_ctx* ctx, const LatticeSetup& s, float* d_values, dcsg_lattice_params& lp);
 
@@ -287,9 +292,9 @@ public:
         cv_.notify_all();
     }
     // soup: 9 floats per triangle; plyRows / stlRecords: where the rows of the run's first triangle go in the file image;
-    // fdPly / fdStl (-1: none) + offsets: where they go in the files
+    // fdPly / fdStl (-1: none) + offsets: where they go in the files; acb: STL records list the corners A, C, B (stl_words)
     void submit_expand(const float* soup, uint64_t tris, uint8_t* plyRows, uint8_t* stlRecords, int fdPly, uint64_t offsetPly, int fdStl,
-                       uint64_t offsetStl) {
+                       uint64_t offsetStl, bool acb) {
         if (!tris) return;
         const uint64_t piece = 32768;
         std::lock_guard<std::mutex> g(m_);
@@ -298,6 +303,7 @@ public:
             job.soup = soup + done * 9; job.tris = std::min(piece, tris - done);
             job.plyRows = plyRows + done * 72; job.stlRecords = stlRecords + done * 50;
             job.fd = fdPly; job.offset = offsetPly + done * 72; job.fdStl = fdStl; job.offsetStl = offsetStl + done * 50;
+            job.acb = acb;
             jobs_.push_back(job);
         }
         cv_.notify_all();
@@ -315,15 +321,17 @@ public:
     // The rows are written once and read by nobody on this core (the file writers / the caller come later): non-temporal
     // stores keep the host from first READING every destination line (a plain store to uncached memory costs a
     // read-for-ownership), which matters because host memory traffic -- DMA writes included -- is what bounds the export.
-    static void stl_words(const float* s, uint32_t rec[12]) {
+    // acb: the corners in the order A, C, B -- an outward-wound mesh, which the (x, z, y) axis order would otherwise mirror
+    static void stl_words(const float* s, uint32_t rec[12], bool acb) {
         rec[0] = rec[1] = rec[2] = 0u;
         for (int v = 0; v < 3; v++) {
-            memcpy(&rec[3 + v * 3 + 0], &s[v * 3 + 0], 4);
-            memcpy(&rec[3 + v * 3 + 1], &s[v * 3 + 2], 4);
-            memcpy(&rec[3 + v * 3 + 2], &s[v * 3 + 1], 4);
+            const float* c = s + (acb && v ? 3 - v : v) * 3;
+            memcpy(&rec[3 + v * 3 + 0], &c[0], 4);
+            memcpy(&rec[3 + v * 3 + 1], &c[2], 4);
+            memcpy(&rec[3 + v * 3 + 2], &c[1], 4);
         }
     }
-    static void expand_rows(const float* soup, uint64_t tris, uint8_t* plyRows, uint8_t* stlRecords) {
+    static void expand_rows(const float* soup, uint64_t tris, uint8_t* plyRows, uint8_t* stlRecords, bool acb) {
         long long* rows = reinterpret_cast<long long*>(plyRows);    // 72-byte rows in a 256-byte aligned image: 8-byte aligned
         for (uint64_t i = 0; i < tris; i++) {
             const float* s = soup + i * 9;
@@ -339,8 +347,8 @@ public:
         if ((reinterpret_cast<uintptr_t>(stlRecords) & 3u) == 0) {
             for (; i + 2 <= tris; i += 2) {
                 uint32_t a[12], b[12];
-                stl_words(soup + i * 9, a);
-                stl_words(soup + (i + 1) * 9, b);
+                stl_words(soup + i * 9, a, acb);
+                stl_words(soup + (i + 1) * 9, b, acb);
                 int* out = reinterpret_cast<int*>(stlRecords + i * 50);
                 for (int k = 0; k < 12; k++) _mm_stream_si32(out + k, (int)a[k]);
                 _mm_stream_si32(out + 12, (int)(b[0] << 16));                   // attribute of the first (0) | low half of b[0]
@@ -350,7 +358,7 @@ public:
         }
         for (; i < tris; i++) {
             uint32_t rec[12];
-            stl_words(soup + i * 9, rec);
+            stl_words(soup + i * 9, rec, acb);
             uint8_t* r = stlRecords + i * 50;
             memcpy(r, rec, 48);
             r[48] = r[49] = 0;
@@ -361,6 +369,7 @@ private:
     struct Job {
         int fd = -1; const uint8_t* data = nullptr; size_t size = 0; uint64_t offset = 0;
         const float* soup = nullptr; uint64_t tris = 0; uint8_t* plyRows = nullptr; uint8_t* stlRecords = nullptr; int fdStl = -1; uint64_t offsetStl = 0;
+        bool acb = false;
     };
     bool write_all(int fd, const uint8_t* data, size_t size, uint64_t offset) {
         size_t done = 0;
@@ -382,7 +391,7 @@ private:
                 jobs_.pop_front();
             }
             if (job.soup) {
-                expand_rows(job.soup, job.tris, job.plyRows, job.stlRecords);
+                expand_rows(job.soup, job.tris, job.plyRows, job.stlRecords, job.acb);
                 if (job.fd >= 0 && !write_all(job.fd, job.plyRows, job.tris * 72, job.offset)) failed_ = true;
                 if (job.fdStl >= 0 && !write_all(job.fdStl, job.stlRecords, job.tris * 50, job.offsetStl)) failed_ = true;
             } else if (!write_all(job.fd, job.data, job.size, job.offset)) {
@@ -416,6 +425,11 @@ struct MeshStorage {        // owned by a dcsg_mesh through `reserved`
     // one run starting at the caller's first_triangle.  (Adaptive slabs: one run per octree level.)
     struct Run { uint64_t local, count, global; };
     std::vector<Run> runs;
+    // Outward winding (dcsg_mesh_orient).  cellUnit: consecutive triangles per table triangle of a cell (1, or the 3p - 2 of a
+    // retopologized strip); set by the extraction and, unlike unitTriangles, kept by the weld.  0 = the cells do not describe
+    // the triangles.  oriented: the triangles face outwards; the STL writers then list the corners A, C, B.
+    uint64_t cellUnit = 0;
+    bool oriented = false;
 };
 
 

@@ -571,30 +571,33 @@ __global__ void __launch_bounds__(kThreads) k_cleanup(const dcsg_cleanup_params 
 
 // ---------------------------------------------------------------------------------------------
 // file bodies.  STL record (reference utils.hpp:59-99): normal (0,0,0), A, B, C each as (x, z, y),
-// uint16 0 = 50 bytes.  Two records = 100 bytes = 25 aligned words per thread.
+// uint16 0 = 50 bytes.  Two records = 100 bytes = 25 aligned words per thread.  kACB: A, C, B instead -- the records of an
+// outward-wound mesh, whose winding the (x, z, y) axis order would otherwise mirror
+template <bool kACB>
 __device__ __forceinline__ void stl_record_words(const float* v, const uint32_t* tri, uint32_t f[12]) {
     f[0] = f[1] = f[2] = 0u;
 #pragma unroll
     for (int k = 0; k < 3; ++k) {
-        const float* q = v + (uint64_t)tri[k] * 3;
+        const float* q = v + (uint64_t)tri[kACB && k ? 3 - k : k] * 3;
         f[3 + k * 3 + 0] = __float_as_uint(q[0]);
         f[3 + k * 3 + 1] = __float_as_uint(q[2]);
         f[3 + k * 3 + 2] = __float_as_uint(q[1]);
     }
 }
 
+template <bool kACB>
 __global__ void __launch_bounds__(kThreads) k_format_stl(const float* __restrict__ v, const uint32_t* __restrict__ tris,
                                                          uint64_t n, uint8_t* __restrict__ out) {
     const uint64_t pair = (uint64_t)blockIdx.x * kThreads + threadIdx.x;
     const uint64_t t0 = pair * 2;
     if (t0 >= n) return;
     uint32_t a[12], b[12];
-    stl_record_words(v, tris + t0 * 3, a);
+    stl_record_words<kACB>(v, tris + t0 * 3, a);
     uint32_t* o = reinterpret_cast<uint32_t*>(out + t0 * 50);
 #pragma unroll
     for (int i = 0; i < 12; ++i) o[i] = a[i];
     if (t0 + 1 < n) {
-        stl_record_words(v, tris + (t0 + 1) * 3, b);
+        stl_record_words<kACB>(v, tris + (t0 + 1) * 3, b);
         o[12] = b[0] << 16;                                    // attribute of A (0) | low half of b[0]
 #pragma unroll
         for (int i = 1; i < 12; ++i) o[12 + i] = (b[i - 1] >> 16) | (b[i] << 16);
@@ -946,6 +949,33 @@ __global__ void __launch_bounds__(kThreads) k_weld_remap(uint32_t* __restrict__ 
     if (k < count) tris[k] = newId[rep[tris[k]]];
 }
 
+// ---------------------------------------------------------------------------------------------
+// outward winding (dcsg_launch_orient): per cell, its triangle count (table triangles x unit), an exclusive scan, then one
+// thread per cell swaps corners 1 and 2 of the triangles of its flagged table slots
+__global__ void __launch_bounds__(kThreads) k_orient_count(const uint8_t* __restrict__ masks, uint64_t n, const uint8_t* __restrict__ triCount,
+                                                           uint32_t unit, uint32_t* __restrict__ count) {
+    const uint64_t i = (uint64_t)blockIdx.x * kThreads + threadIdx.x;
+    if (i < n) count[i] = (uint32_t)__ldg(&triCount[masks[i]]) * unit;
+}
+
+__global__ void __launch_bounds__(kThreads) k_orient_apply(const dcsg_orient_params p, const uint32_t* __restrict__ first) {
+    const uint64_t i = (uint64_t)blockIdx.x * kThreads + threadIdx.x;
+    if (i >= p.numCells) return;
+    const uint32_t mask = p.cellMasks[i];
+    const uint64_t f = first[i];
+    const uint64_t end = f + (uint64_t)__ldg(&p.triCount[mask]) * p.unit;
+    if (i == p.numCells - 1) *p.total = (uint32_t)end;
+    if (end > p.numTriangles) return;                   // cells that do not match the triangles (the caller fails the call)
+    for (uint32_t flip = __ldg(&p.triFlip[mask]); flip; flip &= flip - 1) {
+        uint32_t* tri = p.triangles + (f + (uint64_t)(__ffs(flip) - 1) * p.unit) * 3;
+        for (uint32_t c = 0; c < p.unit; ++c, tri += 3) {
+            const uint32_t b = tri[1];
+            tri[1] = tri[2];
+            tri[2] = b;
+        }
+    }
+}
+
 struct WeldMax {
     __device__ __forceinline__ uint32_t operator()(uint32_t a, uint32_t b) const { return a > b ? a : b; }
 };
@@ -979,6 +1009,20 @@ struct WeldLayout {
     }
 };
 
+// Scratch of the orientation: per-cell counts and their exclusive prefix, then cub's temporary storage
+struct OrientLayout {
+    size_t count, first, temp, tempBytes, total;
+    explicit OrientLayout(uint64_t n) {
+        auto align = [](size_t b) { return (b + 255) & ~(size_t)255; };
+        count = 0;
+        first = align(n * 4);
+        temp = first + align(n * 4);
+        tempBytes = 0;
+        cub::DeviceScan::ExclusiveSum(nullptr, tempBytes, (uint32_t*)nullptr, (uint32_t*)nullptr, (long long)n);
+        total = temp + align(tempBytes);
+    }
+};
+
 }  // namespace
 
 // persistent grids: `ctas` CTAs (the host passes a multiple of the SM count), never more than there can be tiles
@@ -1007,8 +1051,10 @@ void dcsg_launch_worklists(const dcsg_worklist_params& p, cudaStream_t s) {
     k_worklist_fill<<<tiles, kThreads, 0, s>>>(p, tiles);
 }
 void dcsg_launch_cleanup(const dcsg_cleanup_params& p, int ctas, cudaStream_t s) { k_cleanup<<<ctas, kThreads, 0, s>>>(p); }
-void dcsg_launch_format_stl(const float* v, const uint32_t* t, uint64_t n, uint8_t* out, cudaStream_t s) {
-    if (n) k_format_stl<<<blocks_for((n + 1) / 2, kThreads), kThreads, 0, s>>>(v, t, n, out);
+void dcsg_launch_format_stl(const float* v, const uint32_t* t, uint64_t n, uint8_t* out, bool acb, cudaStream_t s) {
+    if (!n) return;
+    if (acb) k_format_stl<true><<<blocks_for((n + 1) / 2, kThreads), kThreads, 0, s>>>(v, t, n, out);
+    else k_format_stl<false><<<blocks_for((n + 1) / 2, kThreads), kThreads, 0, s>>>(v, t, n, out);
 }
 void dcsg_launch_format_ply_vertices(const float* v, const uint32_t* t, uint64_t n, double* out, cudaStream_t s) {
     if (n) k_format_ply_vertices<<<blocks_for(n * 3, kThreads), kThreads, 0, s>>>(v, t, n, out);
@@ -1088,5 +1134,23 @@ cudaError_t dcsg_launch_weld(const dcsg_weld_params& p, cudaStream_t s) {
     if ((e = cub::DeviceScan::ExclusiveSum(temp, tempBytes, first, newId, items, s)) != cudaSuccess) return e;
     k_weld_compact<<<blocks, kThreads, 0, s>>>(p.vertices, p.normals, n, first, newId, p.outVertices, p.outNormals, p.unique);
     if (p.numTriangles) k_weld_remap<<<blocks_for(p.numTriangles * 3, kThreads), kThreads, 0, s>>>(p.triangles, p.numTriangles * 3, rep, newId);
+    return cudaGetLastError();
+}
+
+size_t dcsg_orient_scratch_bytes(uint64_t n) { return OrientLayout(n).total; }
+
+cudaError_t dcsg_launch_orient(const dcsg_orient_params& p, cudaStream_t s) {
+    const uint64_t n = p.numCells;
+    if (!n) return cudaMemsetAsync(p.total, 0, 4, s);
+    const OrientLayout l(n);
+    uint8_t* w = static_cast<uint8_t*>(p.scratch);
+    uint32_t* count = reinterpret_cast<uint32_t*>(w + l.count);
+    uint32_t* first = reinterpret_cast<uint32_t*>(w + l.first);
+    size_t tempBytes = l.tempBytes;
+    const uint32_t blocks = blocks_for(n, kThreads);
+    k_orient_count<<<blocks, kThreads, 0, s>>>(p.cellMasks, n, p.triCount, p.unit, count);
+    cudaError_t e = cub::DeviceScan::ExclusiveSum(w + l.temp, tempBytes, count, first, (long long)n, s);
+    if (e != cudaSuccess) return e;
+    k_orient_apply<<<blocks, kThreads, 0, s>>>(p, first);
     return cudaGetLastError();
 }

@@ -260,6 +260,24 @@ int  dcsg_mesh_weld(dcsg_ctx* ctx, dcsg_mesh* mesh);
 /* The indexed PLY of a mesh as it is (no projection); flags & DCSG_PLY_NORMALS needs d_normals.  No reference counterpart. */
 int  dcsg_write_ply_indexed(dcsg_ctx* ctx, const dcsg_mesh* mesh, int flags, const char* path);
 
+/* ---- outward winding (no reference counterpart: the reference's lookup table winds 399 of its 820 triangles inwards, and its
+ * STL records carry zero normals, so its files mix both windings; DESIGN.md 7c) ----------------------------------------------
+ * dcsg_mesh_orient swaps corners 1 and 2 of every inward-facing triangle, in place on the device: afterwards every triangle
+ * (A, B, C) has (B - A) x (C - A) pointing out of the solid.  Which triangles face inwards follows from the cell's corner mask
+ * and the triangle's slot in the table row alone.  Vertices, normals, cells and the triangle order are untouched; host copies
+ * (copy_to_host) are refreshed; a second call is a no-op.  Works before and after dcsg_mesh_weld and on the `local` mesh of
+ * dcsg_extract_sharded; a mesh the library does not own or without cell masks (the borrowed `whole` of a gather) is refused
+ * with DCSG_ERR_INVALID.  Every writer reads the corners through d_triangles; the STL writers of an oriented mesh list the
+ * corners A, C, B, because the records store each corner as (x, z, y) (reference utils.hpp:59-99), which mirrors the mesh.
+ * The files are then no longer the reference's bytes. */
+int  dcsg_mesh_orient(dcsg_ctx* ctx, dcsg_mesh* mesh);
+
+/* Per-context options of the four dcsg_export* calls (like the progress callback).  DCSG_EXPORT_OUTWARD: dcsg_mesh_orient on the
+ * (slab's) mesh right after the extraction, so that every file the export writes is outward-wound.  0, the default, writes
+ * the reference's bytes. */
+#define DCSG_EXPORT_OUTWARD 1
+int  dcsg_set_export_flags(dcsg_ctx* ctx, int flags);
+
 typedef struct dcsg_export_report {
     float    box[6];
     uint64_t num_vertices, num_triangles, num_cells;
