@@ -7,6 +7,9 @@
                                                                        normals; not the reference's format)
     ... export ... --outward                                           every triangle wound to face out of the solid (any of
                                                                        the files above; not the reference's bytes)
+    python -m designcsg_b200 inspect SCENE_DIR|DESIGN.py [--level L] [--outward] [--components]
+                                                                       one JSON line: edge topology, shells, area, volume,
+                                                                       centroid and extents of the mesh --ply-indexed writes
     torchrun --nproc-per-node G -m designcsg_b200 export ...          z-slab sharded over G GPUs (dcsg_export_sharded; the
                                                                        same export from a C host: tools/dcsg_mgpu.c)
 """
@@ -45,6 +48,21 @@ def _export_config(scene):
     return cfg
 
 
+def _export_levels(scene, level_override):
+    """(exportConfig.txt lines or None, search diameter, projection steps, minimum / maximum octree level, grid level,
+    complex-surface threshold) of an export; level_override L > 0 = uniform lattice of 2^L cells per side."""
+    cfg = _export_config(scene)
+    if cfg is None and not level_override:
+        raise SystemExit("%s has no exportConfig.txt (the design never called setExportConfig): pass --level L" % scene)
+    # exportConfig.txt lines 1-6: search diameter, minimum / maximum octree level, grid level, complex-surface threshold,
+    # projection steps
+    search, steps = (float(cfg[0]), int(cfg[5])) if cfg else (10.0, 50)
+    lo, hi, level, threshold = (int(cfg[1]), int(cfg[2]), int(cfg[3]), float(cfg[4])) if cfg else (0, 0, 0, float(np.pi / 4))
+    if level_override:
+        lo = hi = level = level_override
+    return cfg, search, steps, lo, hi, level, threshold
+
+
 def cmd_export(args):
     from . import api, build
     world = int(os.environ.get("WORLD_SIZE", "1"))
@@ -62,16 +80,7 @@ def cmd_export(args):
                              "spans the GPUs' slabs")
     build.build()                       # serialised across the ranks of a node by a file lock; the first one compiles
     scene = _scene_dir(args.scene)
-    cfg = _export_config(scene)
-    if cfg is None and not args.level:
-        raise SystemExit("%s has no exportConfig.txt (the design never called setExportConfig): pass --level L" % scene)
-    # exportConfig.txt lines 1-6: search diameter, minimum / maximum octree level, grid level, complex-surface threshold,
-    # projection steps; --level L = uniform lattice of 2^L cells per side
-    search, steps = (float(cfg[0]), int(cfg[5])) if cfg else (10.0, 50)
-    lo, hi, level, threshold = (int(cfg[1]), int(cfg[2]), int(cfg[3]), float(cfg[4])) if cfg else (0, 0, 0, float(np.pi / 4))
-    if args.level:
-        lo = hi = level = args.level
-    uniform = lo >= level and hi == level
+    cfg, search, steps, lo, hi, level, threshold = _export_levels(scene, args.level)
     t0 = time.perf_counter()
     ctx = api.Context(local)
     ctx.build(scene)
@@ -128,6 +137,34 @@ def cmd_export(args):
         print(json.dumps(report))
 
 
+def cmd_inspect(args):
+    """The report of dcsg_mesh_inspect on the mesh `export --ply-indexed` writes with the same options: extraction (the
+    export's levels, threshold and retopologize), --outward orientation, the weld of adaptive levels, the projection."""
+    from . import api, build
+    if int(os.environ.get("WORLD_SIZE", "1")) > 1:
+        raise SystemExit("inspect runs on one GPU: the mesh of a sharded export is never gathered; run it without torchrun")
+    build.build()
+    scene = _scene_dir(args.scene)
+    _, search, steps, lo, hi, level, threshold = _export_levels(scene, args.level)
+    ctx = api.Context(int(os.environ.get("LOCAL_RANK", "0")))
+    ctx.build(scene)
+    mesh = ctx.extract(ctx.bbox(search), level, copy_to_host=False, min_level=lo, max_level=hi, complex_threshold=threshold,
+                       retopologize=True, defer_projection=True)
+    if args.outward:
+        mesh.orient()
+    if not (lo >= level and hi == level):
+        mesh.weld()
+    ctx.project(mesh, steps)
+    report = mesh.inspect(components=args.components)
+    for name in ("component_triangles", "component_area", "component_signed_volume"):
+        if name in report:
+            report[name] = report[name].tolist()
+    report.update(scene=scene, octree_levels=[lo, hi, level], gd_steps=steps, outward=bool(args.outward))
+    mesh.free()
+    ctx.close()
+    print(json.dumps(report))
+
+
 def main():
     ap = argparse.ArgumentParser(prog="python -m designcsg_b200")
     sub = ap.add_subparsers(dest="cmd", required=True)
@@ -148,6 +185,12 @@ def main():
     e.add_argument("--outward", action="store_true", help="wind every triangle to face out of the solid (dcsg_mesh_orient) in "
                    "whichever files are written; the files are then not the reference's bytes, whose winding is mixed")
     e.set_defaults(fn=cmd_export)
+    i = sub.add_parser("inspect", help="report on the mesh `export --ply-indexed` would write (one JSON line)")
+    i.add_argument("scene", help="scene directory or design script")
+    i.add_argument("--level", type=int, default=0, help="uniform lattice of 2^L cells per side (default: exportConfig.txt's levels)")
+    i.add_argument("--outward", action="store_true", help="orient the mesh first, as export --outward does")
+    i.add_argument("--components", action="store_true", help="add per-shell triangle counts, areas and signed volumes")
+    i.set_defaults(fn=cmd_inspect)
     args = ap.parse_args()
     args.fn(args)
 

@@ -61,6 +61,15 @@ class ShardInfo(ctypes.Structure):
                 ("total_triangles", ctypes.c_uint64), ("total_cells", ctypes.c_uint64)]
 
 
+class MeshReport(ctypes.Structure):
+    _fields_ = [(name, ctypes.c_uint64) for name in (
+                    "num_vertices", "num_triangles", "unreferenced_vertices", "nonfinite_vertices", "degenerate_triangles",
+                    "zero_area_triangles", "nonfinite_triangles", "edges", "boundary_edges", "manifold_edges", "nonmanifold_edges",
+                    "misoriented_edges", "components")] + \
+               [("area", ctypes.c_double), ("signed_volume", ctypes.c_double), ("centroid", ctypes.c_double * 3),
+                ("bbox_min", ctypes.c_float * 3), ("bbox_max", ctypes.c_float * 3)]
+
+
 PROGRESS_STATES = ("IDLE", "ESTIMATING_BOUNDING_BOX", "PERFORMING_CMS", "RETOPOLOGIZING", "GRADIENT_DESCENT", "WRITING_STL",
                    "WRITING_PLY", "COMPLETE")                   # dcsg.h DCSG_PROGRESS_*, reference DesignCSG.cpp:603-614
 PROGRESS_FN = ctypes.CFUNCTYPE(None, ctypes.c_void_p, ctypes.c_int, ctypes.c_uint64, ctypes.c_uint64)
@@ -143,6 +152,8 @@ def load_library():
     lib.dcsg_export_sharded_indexed.argtypes = [vp, vp, cp, ci, ci, cp, ctypes.POINTER(ExportReport)]
     lib.dcsg_mesh_orient.argtypes = [vp, ctypes.POINTER(MeshStruct)]
     lib.dcsg_set_export_flags.argtypes = [vp, ci]
+    lib.dcsg_mesh_inspect.argtypes = [vp, ctypes.POINTER(MeshStruct), ctypes.POINTER(MeshReport), ctypes.c_uint64, _u64p,
+                                      ctypes.POINTER(ctypes.c_double), ctypes.POINTER(ctypes.c_double)]
     _lib = lib
     return lib
 
@@ -310,6 +321,27 @@ class Mesh:
         Vertices, cells and triangle order stay; the host arrays are refreshed when the mesh was copied to the host; a second
         call changes nothing.  The STL writers then list the corners A, C, B (the files are no longer the reference's bytes)."""
         self._ctx._check(self._ctx.lib.dcsg_mesh_orient(self._ctx.h, ctypes.byref(self.c)))
+
+    def inspect(self, components=False):
+        """dcsg_mesh_inspect: the mesh's report as a dict -- edge topology (boundary, manifold, non-manifold, misoriented edges),
+        shells, degenerate / zero-area / non-finite triangles, area, signed volume, centroid and float extents.  components=True
+        adds the per-shell `component_triangles`, `component_area` and `component_signed_volume` arrays (shells in the order of
+        their smallest vertex id).  Reads the device arrays; changes nothing."""
+        rep = MeshReport()
+        cap = self.num_vertices // 3 if components else 0
+        tris, area, vol = np.zeros(cap, np.uint64), np.zeros(cap, np.float64), np.zeros(cap, np.float64)
+        dp = ctypes.POINTER(ctypes.c_double)
+        self._ctx._check(self._ctx.lib.dcsg_mesh_inspect(self._ctx.h, ctypes.byref(self.c), ctypes.byref(rep), cap,
+                                                         tris.ctypes.data_as(_u64p) if cap else None,
+                                                         area.ctypes.data_as(dp) if cap else None, vol.ctypes.data_as(dp) if cap else None))
+        out = {}
+        for name, kind in MeshReport._fields_:
+            v = getattr(rep, name)
+            out[name] = [float(x) for x in v] if hasattr(v, "__len__") else (float(v) if kind is ctypes.c_double else int(v))
+        if components:
+            n = out["components"]
+            out.update(component_triangles=tris[:n], component_area=area[:n], component_signed_volume=vol[:n])
+        return out
 
     def write_ply_indexed(self, path, normals=False):
         """dcsg_write_ply_indexed: binary PLY with shared float vertices (and the mesh's normals) -- not the reference's format."""

@@ -53,7 +53,7 @@ void dcsg_destroy(dcsg_ctx* ctx) {
     cudaSetDevice(ctx->device);
     cudaStreamSynchronize(ctx->stream);
     for (DevBuf* b : {&ctx->pts, &ctx->vals, &ctx->axes, &ctx->sign, &ctx->leaf, &ctx->cfail, &ctx->coarse, &ctx->levels, &ctx->alive, &ctx->vinfo,
-                      &ctx->tiles, &ctx->small, &ctx->lattice_values, &ctx->fmt, &ctx->adapt_emit, &ctx->adapt_snap, &ctx->search_bits, &ctx->project_cursor, &ctx->lists, &ctx->masks, &ctx->soup, &ctx->project_list, &ctx->weld, &ctx->orient})
+                      &ctx->tiles, &ctx->small, &ctx->lattice_values, &ctx->fmt, &ctx->adapt_emit, &ctx->adapt_snap, &ctx->search_bits, &ctx->project_cursor, &ctx->lists, &ctx->masks, &ctx->soup, &ctx->project_list, &ctx->weld, &ctx->orient, &ctx->inspect})
         b->release();
     ctx->pinned.release();
     ctx->pinned_small.release();

@@ -3,7 +3,7 @@
 // bounding box, slab plan, preview; host_extract.cu: lattice passes and dcsg_extract; host_files.cu: byte-exact
 // files, the projection / format / copy / write pipeline, the one driver behind dcsg_export, dcsg_export_sharded,
 // dcsg_export_indexed and dcsg_export_sharded_indexed; host_indexed.cu: the weld and the indexed PLY's pipeline;
-// host_comm.cu: the communicator and the sharded search and extraction).  Not part of the ABI (include/dcsg.h is).
+// host_inspect.cu: the mesh report; host_comm.cu: the communicator and the sharded search and extraction).  Not part of the ABI (include/dcsg.h is).
 #pragma once
 #include <cuda_runtime.h>
 #include <nvrtc.h>
@@ -197,7 +197,8 @@ struct dcsg_ctx {
     dcsg_host::DevBuf pts, vals, axes, sign, leaf, cfail, coarse, levels, alive, vinfo, tiles, small, lattice_values, fmt,
            adapt_emit, adapt_snap, search_bits, project_cursor, project_list, lists, masks, soup,
            weld,                    // dcsg_mesh_weld: sort / scan scratch, then the compacted vertices and normals
-           orient;                  // dcsg_mesh_orient: per-cell counts, their prefix and the scan's scratch
+           orient,                  // dcsg_mesh_orient: per-cell counts, their prefix and the scan's scratch
+           inspect;                 // dcsg_mesh_inspect: sort / reduction scratch, the component runs, the totals
     dcsg_host::HostBuf pinned, pinned_small, pinned_soup;
     // sparse extraction: `leaf` (as leafAlive) and `alive` are all-zero between extractions -- every sparse
     // extraction zeroes the words it wrote (dcsg_launch_cleanup); anything else that writes them clears this flag

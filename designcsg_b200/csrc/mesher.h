@@ -152,6 +152,45 @@ struct dcsg_orient_params {
 size_t dcsg_orient_scratch_bytes(uint64_t numCells);
 cudaError_t dcsg_launch_orient(const dcsg_orient_params& p, cudaStream_t s);
 
+// Mesh inspection (dcsg_mesh_inspect; definitions in include/dcsg.h and DESIGN.md 7d).  Radix sorts, run-length reductions and
+// reductions of cub plus map kernels, every floating-point sum a cub reduction in a fixed order: the same bits on every run.
+// A triangle is degenerate when two of its ids are equal; ids must be < numVertices (dcsg_launch_inspect_check first).
+struct dcsg_inspect_vertex_sums {
+    uint64_t referenced, nonfinite, roots;      // roots: referenced vertices that are their component's smallest id
+    float lo[3], hi[3];                         // over referenced finite vertices; +Inf / -Inf without any
+};
+struct dcsg_inspect_triangle_sums {
+    uint64_t degenerate, zeroArea, nonfinite;
+    double area, volume, moment[3];             // moment: sum of vol_t * (a + b + c) per axis
+};
+struct dcsg_inspect_edge_sums {
+    uint64_t edges, boundary, manifold, nonmanifold, misoriented;
+};
+struct dcsg_inspect_component {                 // one run of the components' segmented reduction
+    uint64_t triangles;
+    double area, volume;
+};
+struct dcsg_inspect_totals {
+    dcsg_inspect_vertex_sums v;
+    dcsg_inspect_triangle_sums t;
+    dcsg_inspect_edge_sums e;
+    uint64_t componentRuns;                     // components, plus one run for the degenerate triangles if there are any
+    uint32_t badIds;                            // dcsg_launch_inspect_check: 1 = some id >= numVertices
+};
+struct dcsg_inspect_params {
+    const float* vertices;
+    const uint32_t* triangles;
+    uint64_t numVertices;                       // < 2^32
+    uint64_t numTriangles;                      // > 0
+    void* scratch;                              // dcsg_inspect_scratch_bytes(numVertices, numTriangles) bytes of device memory
+    dcsg_inspect_totals* totals;                // device
+    dcsg_inspect_component* components;         // device, numTriangles entries: components in the order of their smallest id
+};
+size_t dcsg_inspect_scratch_bytes(uint64_t numVertices, uint64_t numTriangles);
+// reads the triangles only: totals->badIds
+cudaError_t dcsg_launch_inspect_check(const dcsg_inspect_params& p, cudaStream_t s);
+cudaError_t dcsg_launch_inspect(const dcsg_inspect_params& p, cudaStream_t s);
+
 // ---- adaptive octree mode (mesher_kernels.cu "adaptive") ----------------------------------------------
 struct dcsg_adapt_emit_params {
     dcsg_grid g;                    // the slab of sample planes the sign bitmap covers (z0 = its first plane)

@@ -24,7 +24,12 @@
 
 #include <algorithm>
 #include <cub/device/device_radix_sort.cuh>
+#include <cub/device/device_reduce.cuh>
 #include <cub/device/device_scan.cuh>
+#include <cub/device/device_segmented_reduce.cuh>
+#include <cub/device/device_select.cuh>
+#include <thrust/iterator/counting_iterator.h>
+#include <thrust/iterator/transform_iterator.h>
 
 namespace {
 
@@ -1023,6 +1028,298 @@ struct OrientLayout {
     }
 };
 
+// ---------------------------------------------------------------------------------------------
+// mesh inspection (dcsg_launch_inspect).  Triangles t, half-edges 3t + e, vertices v.
+// ---------------------------------------------------------------------------------------------
+constexpr uint64_t kNoEdge = ~0ull;                     // half-edge key of a degenerate triangle: sorts after every real key
+constexpr uint32_t kNoLabel = ~0u;                      // component label of a degenerate triangle
+
+__device__ __forceinline__ bool inspect_degenerate(uint32_t a, uint32_t b, uint32_t c) { return a == b || b == c || a == c; }
+
+__global__ void __launch_bounds__(kThreads) k_inspect_check(const uint32_t* __restrict__ tris, uint64_t count, uint64_t numVertices,
+                                                            uint32_t* __restrict__ bad) {
+    const uint64_t k = (uint64_t)blockIdx.x * kThreads + threadIdx.x;
+    if (k < count && tris[k] >= numVertices) atomicOr(bad, 1u);
+}
+
+__global__ void __launch_bounds__(kThreads) k_inspect_init(uint64_t n, uint32_t* __restrict__ parent, uint8_t* __restrict__ ref) {
+    const uint64_t v = (uint64_t)blockIdx.x * kThreads + threadIdx.x;
+    if (v >= n) return;
+    parent[v] = (uint32_t)v;
+    ref[v] = 0;
+}
+
+// Union-find whose parents only ever decrease (parent[v] <= v): a root is the smallest id of its tree.  Only roots are
+// written by atomicCAS, only non-roots by the path halving's plain stores, and both store an ancestor, so every interleaving
+// leaves the same partition, and the final roots -- the components' smallest ids -- do not depend on the schedule.
+__device__ __forceinline__ uint32_t uf_find(uint32_t* p, uint32_t x) {
+    volatile uint32_t* vp = p;
+    uint32_t cur = vp[x];
+    if (cur == x) return x;
+    uint32_t prev = x, next;
+    while (cur > (next = vp[cur])) {
+        vp[prev] = next;
+        prev = cur;
+        cur = next;
+    }
+    return cur;
+}
+
+__device__ __forceinline__ void uf_unite(uint32_t* p, uint32_t a, uint32_t b) {
+    a = uf_find(p, a);
+    b = uf_find(p, b);
+    while (a != b) {
+        if (a > b) { const uint32_t t = a; a = b; b = t; }
+        const uint32_t old = atomicCAS(&p[b], b, a);     // hook the larger root under the smaller one
+        if (old == b) return;
+        b = uf_find(p, old);                              // b was hooked meanwhile: go on from its new root
+        a = uf_find(p, a);
+    }
+}
+
+// per triangle: its half-edge keys min << 32 | max with the direction bit (a < b), the referenced marks, the unions
+__global__ void __launch_bounds__(kThreads) k_inspect_triangles(const uint32_t* __restrict__ tris, uint64_t n, uint64_t* __restrict__ keys,
+                                                                uint8_t* __restrict__ fwd, uint8_t* __restrict__ ref, uint32_t* parent) {
+    const uint64_t t = (uint64_t)blockIdx.x * kThreads + threadIdx.x;
+    if (t >= n) return;
+    const uint32_t id[3] = {tris[t * 3], tris[t * 3 + 1], tris[t * 3 + 2]};
+    const bool deg = inspect_degenerate(id[0], id[1], id[2]);
+#pragma unroll
+    for (int e = 0; e < 3; ++e) {
+        const uint32_t x = id[e], y = id[e == 2 ? 0 : e + 1];
+        keys[t * 3 + e] = deg ? kNoEdge : ((uint64_t)min(x, y) << 32) | max(x, y);
+        fwd[t * 3 + e] = x < y ? 1 : 0;
+    }
+    if (deg) return;
+    ref[id[0]] = ref[id[1]] = ref[id[2]] = 1;
+    uf_unite(parent, id[0], id[1]);
+    uf_unite(parent, id[0], id[2]);
+}
+
+// Every vertex to its root.  No path halving here: a halving store of another thread could put an older ancestor back over a
+// root this pass has already written.  Each thread writes only its own vertex, and only the root, which no longer changes.
+__global__ void __launch_bounds__(kThreads) k_inspect_flatten(uint64_t n, uint32_t* parent) {
+    const uint64_t v = (uint64_t)blockIdx.x * kThreads + threadIdx.x;
+    if (v >= n) return;
+    volatile uint32_t* vp = parent;
+    uint32_t r = (uint32_t)v, next;
+    while ((next = vp[r]) != r) r = next;
+    vp[v] = r;
+}
+
+__global__ void __launch_bounds__(kThreads) k_inspect_labels(const uint32_t* __restrict__ tris, uint64_t n, const uint32_t* __restrict__ parent,
+                                                             uint32_t* __restrict__ label, uint32_t* __restrict__ index) {
+    const uint64_t t = (uint64_t)blockIdx.x * kThreads + threadIdx.x;
+    if (t >= n) return;
+    const uint32_t a = tris[t * 3], b = tris[t * 3 + 1], c = tris[t * 3 + 2];
+    label[t] = inspect_degenerate(a, b, c) ? kNoLabel : parent[a];
+    index[t] = (uint32_t)t;
+}
+
+// The shells' sums (dcsg_launch_inspect): the sorted (label, triangle) sequence is cut into pieces at every label change and
+// every kInspectPiece-th item; each piece, then each shell's run of piece partials, is one segment of a segmented reduction --
+// one CTA per segment in a fixed order, unlike a reduction by key, whose look-back combines the partials of a run that spans
+// tiles in an order that depends on the schedule.
+constexpr long long kInspectPiece = 4096;
+using InspectCount = thrust::counting_iterator<long long>;
+
+__global__ void __launch_bounds__(kThreads) k_inspect_piece_heads(const uint32_t* __restrict__ label, uint64_t n, uint8_t* __restrict__ head) {
+    const uint64_t i = (uint64_t)blockIdx.x * kThreads + threadIdx.x;
+    if (i < n) head[i] = i == 0 || label[i] != label[i - 1] || i % kInspectPiece == 0;
+}
+
+// piece q starts a shell's run when its first item's label differs from the previous piece's (flags past the pieces: 0)
+__global__ void __launch_bounds__(kThreads) k_inspect_run_heads(const uint32_t* __restrict__ label, uint64_t n, const long long* __restrict__ pieceBegin,
+                                                                const long long* __restrict__ pieces, uint8_t* __restrict__ head) {
+    const long long q = (long long)blockIdx.x * kThreads + threadIdx.x;
+    if ((uint64_t)q < n) head[q] = q < *pieces && (q == 0 || label[pieceBegin[q]] != label[pieceBegin[q - 1]]);
+}
+
+// end of segment s: the next one's begin, or `total` after the last of *count
+struct InspectSegmentEnd {
+    const long long* begin;
+    const long long* count;
+    long long total;
+    __device__ long long operator()(long long s) const { return s + 1 < *count ? begin[s + 1] : total; }
+};
+using InspectEnds = thrust::transform_iterator<InspectSegmentEnd, InspectCount>;
+
+// exact float minimum / maximum, -0 below +0, so that the order of the reduction cannot show
+__device__ __forceinline__ float min_total(float a, float b) { return (a < b || (a == b && signbit(a))) ? a : b; }
+__device__ __forceinline__ float max_total(float a, float b) { return (a > b || (a == b && !signbit(b))) ? a : b; }
+
+struct InspectVertexTerm {
+    const float* v;
+    const uint8_t* ref;
+    const uint32_t* parent;
+    __device__ dcsg_inspect_vertex_sums operator()(long long i) const {
+        dcsg_inspect_vertex_sums s;
+        const float x = v[i * 3], y = v[i * 3 + 1], z = v[i * 3 + 2];
+        const bool r = ref[i] != 0, finite = isfinite(x) && isfinite(y) && isfinite(z), use = r && finite;
+        s.referenced = r;
+        s.nonfinite = r && !finite;
+        s.roots = r && parent[i] == (uint32_t)i;
+        s.lo[0] = use ? x : INFINITY; s.lo[1] = use ? y : INFINITY; s.lo[2] = use ? z : INFINITY;
+        s.hi[0] = use ? x : -INFINITY; s.hi[1] = use ? y : -INFINITY; s.hi[2] = use ? z : -INFINITY;
+        return s;
+    }
+};
+struct InspectVertexSum {
+    __device__ dcsg_inspect_vertex_sums operator()(const dcsg_inspect_vertex_sums& a, const dcsg_inspect_vertex_sums& b) const {
+        dcsg_inspect_vertex_sums s;
+        s.referenced = a.referenced + b.referenced;
+        s.nonfinite = a.nonfinite + b.nonfinite;
+        s.roots = a.roots + b.roots;
+        for (int c = 0; c < 3; ++c) { s.lo[c] = min_total(a.lo[c], b.lo[c]); s.hi[c] = max_total(a.hi[c], b.hi[c]); }
+        return s;
+    }
+};
+
+// The per-triangle terms, one fixed sequence of double operations (the library is compiled with -fmad=false): DESIGN.md 7d.
+struct InspectTriangleTerm {
+    const float* v;
+    const uint32_t* tris;
+    __device__ dcsg_inspect_triangle_sums operator()(long long t) const {
+        dcsg_inspect_triangle_sums s = {};
+        const uint32_t ia = tris[t * 3], ib = tris[t * 3 + 1], ic = tris[t * 3 + 2];
+        if (inspect_degenerate(ia, ib, ic)) { s.degenerate = 1; return s; }
+        const float* fa = v + (uint64_t)ia * 3;
+        const float* fb = v + (uint64_t)ib * 3;
+        const float* fc = v + (uint64_t)ic * 3;
+        bool finite = true;
+        for (int c = 0; c < 3; ++c) finite = finite && isfinite(fa[c]) && isfinite(fb[c]) && isfinite(fc[c]);
+        if (!finite) { s.nonfinite = 1; return s; }
+        const double ax = fa[0], ay = fa[1], az = fa[2], bx = fb[0], by = fb[1], bz = fb[2], cx = fc[0], cy = fc[1], cz = fc[2];
+        const double ux = bx - ax, uy = by - ay, uz = bz - az, wx = cx - ax, wy = cy - ay, wz = cz - az;
+        const double nx = uy * wz - uz * wy, ny = uz * wx - ux * wz, nz = ux * wy - uy * wx;
+        s.zeroArea = nx == 0.0 && ny == 0.0 && nz == 0.0;
+        s.area = 0.5 * sqrt((nx * nx + ny * ny) + nz * nz);
+        s.volume = ((ax * (by * cz - bz * cy) + ay * (bz * cx - bx * cz)) + az * (bx * cy - by * cx)) / 6.0;
+        s.moment[0] = s.volume * ((ax + bx) + cx);
+        s.moment[1] = s.volume * ((ay + by) + cy);
+        s.moment[2] = s.volume * ((az + bz) + cz);
+        return s;
+    }
+};
+struct InspectTriangleSum {
+    __device__ dcsg_inspect_triangle_sums operator()(const dcsg_inspect_triangle_sums& a, const dcsg_inspect_triangle_sums& b) const {
+        dcsg_inspect_triangle_sums s;
+        s.degenerate = a.degenerate + b.degenerate;
+        s.zeroArea = a.zeroArea + b.zeroArea;
+        s.nonfinite = a.nonfinite + b.nonfinite;
+        s.area = a.area + b.area;
+        s.volume = a.volume + b.volume;
+        for (int c = 0; c < 3; ++c) s.moment[c] = a.moment[c] + b.moment[c];
+        return s;
+    }
+};
+
+// component runs: the triangles of a run, by index, in ascending order (the sort is stable)
+struct InspectComponentTerm {
+    InspectTriangleTerm term;
+    __device__ dcsg_inspect_component operator()(uint32_t t) const {
+        const dcsg_inspect_triangle_sums s = term((long long)t);
+        return dcsg_inspect_component{1, s.area, s.volume};
+    }
+};
+struct InspectComponentSum {
+    __device__ dcsg_inspect_component operator()(const dcsg_inspect_component& a, const dcsg_inspect_component& b) const {
+        return dcsg_inspect_component{a.triangles + b.triangles, a.area + b.area, a.volume + b.volume};
+    }
+};
+
+// half-edge runs: (1 << 32 | direction bit) summed per key = (k half-edges) << 32 | (f of them with a < b)
+struct InspectHalfEdge {
+    __device__ uint64_t operator()(uint8_t forward) const { return (1ull << 32) | forward; }
+};
+struct InspectAdd {
+    __device__ uint64_t operator()(uint64_t a, uint64_t b) const { return a + b; }
+};
+struct InspectEdgeTerm {
+    const uint64_t* key;
+    const uint64_t* packed;
+    const uint64_t* runs;
+    __device__ dcsg_inspect_edge_sums operator()(long long i) const {
+        dcsg_inspect_edge_sums s = {};
+        if ((uint64_t)i >= *runs || key[i] == kNoEdge) return s;
+        const uint64_t k = packed[i] >> 32, f = packed[i] & 0xffffffffull;
+        s.edges = 1;
+        s.boundary = k == 1;
+        s.manifold = k == 2;
+        s.nonmanifold = k >= 3;
+        s.misoriented = k == 2 && f != 1;
+        return s;
+    }
+};
+struct InspectEdgeSum {
+    __device__ dcsg_inspect_edge_sums operator()(const dcsg_inspect_edge_sums& a, const dcsg_inspect_edge_sums& b) const {
+        return dcsg_inspect_edge_sums{a.edges + b.edges, a.boundary + b.boundary, a.manifold + b.manifold, a.nonmanifold + b.nonmanifold,
+                                      a.misoriented + b.misoriented};
+    }
+};
+
+using InspectHalfEdges = thrust::transform_iterator<InspectHalfEdge, const uint8_t*>;
+using InspectComponentTerms = thrust::transform_iterator<InspectComponentTerm, const uint32_t*>;
+
+// bits of the sort keys: ids < n need bitsFor(n) bits, and the sentinels' low bits (all ones) still sort last
+inline int bits_for(uint64_t n) {
+    int b = 1;
+    while (b < 32 && (n >> b)) ++b;
+    return b;
+}
+
+// Scratch of the inspection: half-edge keys and direction bits (sorted copies), the runs' packed counts, union-find parents and
+// referenced marks, triangle labels and indices (sorted copies), the edge run count, then cub's temporary storage
+struct InspectLayout {
+    size_t keysA, keysB, fwdA, fwdB, packed, parent, ref, labelA, labelB, indexA, indexB, head, pieceBegin, runBegin, partial, runs, counts,
+        temp, tempBytes, total;
+    InspectLayout(uint64_t nv, uint64_t nt) {
+        auto align = [](size_t b) { return (b + 255) & ~(size_t)255; };
+        const uint64_t h = nt * 3;
+        size_t o = 0;
+        keysA = o; o += align(h * 8);
+        keysB = o; o += align(h * 8);
+        fwdA = o; o += align(h);
+        fwdB = o; o += align(h);
+        packed = o; o += align(h * 8);
+        parent = o; o += align(nv * 4);
+        ref = o; o += align(nv);
+        labelA = o; o += align(nt * 4);
+        labelB = o; o += align(nt * 4);
+        indexA = o; o += align(nt * 4);
+        indexB = o; o += align(nt * 4);
+        head = o; o += align(nt);
+        pieceBegin = o; o += align(nt * 8);
+        runBegin = o; o += align(nt * 8);
+        partial = o; o += align(nt * sizeof(dcsg_inspect_component));
+        runs = o; o += align(8);
+        counts = o; o += align(16);
+        size_t b[10] = {};
+        const long long hi = (long long)h, ti = (long long)nt, vi = (long long)nv;
+        cub::DeviceRadixSort::SortPairs(nullptr, b[0], (uint64_t*)nullptr, (uint64_t*)nullptr, (uint8_t*)nullptr, (uint8_t*)nullptr, hi);
+        cub::DeviceReduce::ReduceByKey(nullptr, b[1], (uint64_t*)nullptr, (uint64_t*)nullptr, InspectHalfEdges(nullptr, InspectHalfEdge()),
+                                       (uint64_t*)nullptr, (uint64_t*)nullptr, InspectAdd(), hi);
+        cub::DeviceRadixSort::SortPairs(nullptr, b[2], (uint32_t*)nullptr, (uint32_t*)nullptr, (uint32_t*)nullptr, (uint32_t*)nullptr, ti);
+        cub::DeviceSelect::Flagged(nullptr, b[3], InspectCount(0), (const uint8_t*)nullptr, (long long*)nullptr, (long long*)nullptr, ti);
+        const int segs = (int)std::min<uint64_t>(nt, 0x7fffffffull);
+        const InspectEnds ends(InspectCount(0), InspectSegmentEnd{});
+        cub::DeviceSegmentedReduce::Reduce(nullptr, b[7], InspectComponentTerms(nullptr, InspectComponentTerm{}),
+                                           (dcsg_inspect_component*)nullptr, segs, (const long long*)nullptr, ends, InspectComponentSum(),
+                                           dcsg_inspect_component{});
+        cub::DeviceSegmentedReduce::Reduce(nullptr, b[8], (const dcsg_inspect_component*)nullptr, (dcsg_inspect_component*)nullptr, segs,
+                                           (const long long*)nullptr, ends, InspectComponentSum(), dcsg_inspect_component{});
+        cub::DeviceReduce::Reduce(nullptr, b[4], thrust::make_transform_iterator(InspectCount(0), InspectVertexTerm{}),
+                                  (dcsg_inspect_vertex_sums*)nullptr, vi, InspectVertexSum(), dcsg_inspect_vertex_sums{});
+        cub::DeviceReduce::Reduce(nullptr, b[5], thrust::make_transform_iterator(InspectCount(0), InspectTriangleTerm{}),
+                                  (dcsg_inspect_triangle_sums*)nullptr, ti, InspectTriangleSum(), dcsg_inspect_triangle_sums{});
+        cub::DeviceReduce::Reduce(nullptr, b[6], thrust::make_transform_iterator(InspectCount(0), InspectEdgeTerm{}),
+                                  (dcsg_inspect_edge_sums*)nullptr, hi, InspectEdgeSum(), dcsg_inspect_edge_sums{});
+        tempBytes = *std::max_element(b, b + 10);
+        temp = o; o += align(tempBytes);
+        total = o;
+    }
+};
+
 }  // namespace
 
 // persistent grids: `ctas` CTAs (the host passes a multiple of the SM count), never more than there can be tiles
@@ -1152,5 +1449,93 @@ cudaError_t dcsg_launch_orient(const dcsg_orient_params& p, cudaStream_t s) {
     cudaError_t e = cub::DeviceScan::ExclusiveSum(w + l.temp, tempBytes, count, first, (long long)n, s);
     if (e != cudaSuccess) return e;
     k_orient_apply<<<blocks, kThreads, 0, s>>>(p, first);
+    return cudaGetLastError();
+}
+
+size_t dcsg_inspect_scratch_bytes(uint64_t nv, uint64_t nt) { return InspectLayout(nv, nt).total; }
+
+cudaError_t dcsg_launch_inspect_check(const dcsg_inspect_params& p, cudaStream_t s) {
+    cudaError_t e = cudaMemsetAsync(p.totals, 0, sizeof(dcsg_inspect_totals), s);
+    if (e != cudaSuccess) return e;
+    k_inspect_check<<<blocks_for(p.numTriangles * 3, kThreads), kThreads, 0, s>>>(p.triangles, p.numTriangles * 3, p.numVertices, &p.totals->badIds);
+    return cudaGetLastError();
+}
+
+// Edges: the half-edge keys radix-sorted with their direction bits, then one reduction by key gives every edge's (k, f).
+// Components: union-find over the non-degenerate triangles' ids, flattened to the smallest id, then the (label, triangle)
+// pairs radix-sorted (stable: ascending triangles within a label) and summed by two segmented reductions (pieces, then the
+// shells' runs of pieces).  Sums: cub reductions of the per-vertex, per-triangle and per-edge terms.  No floating-point atomics
+// and no floating-point reduction by key: every result is the same bits on every run.
+cudaError_t dcsg_launch_inspect(const dcsg_inspect_params& p, cudaStream_t s) {
+    const uint64_t nv = p.numVertices, nt = p.numTriangles, nh = nt * 3;
+    const InspectLayout l(nv, nt);
+    uint8_t* w = static_cast<uint8_t*>(p.scratch);
+    uint64_t* keysA = reinterpret_cast<uint64_t*>(w + l.keysA);
+    uint64_t* keysB = reinterpret_cast<uint64_t*>(w + l.keysB);
+    uint8_t* fwdA = w + l.fwdA;
+    uint8_t* fwdB = w + l.fwdB;
+    uint64_t* packed = reinterpret_cast<uint64_t*>(w + l.packed);
+    uint32_t* parent = reinterpret_cast<uint32_t*>(w + l.parent);
+    uint8_t* ref = w + l.ref;
+    uint32_t* labelA = reinterpret_cast<uint32_t*>(w + l.labelA);
+    uint32_t* labelB = reinterpret_cast<uint32_t*>(w + l.labelB);
+    uint32_t* indexA = reinterpret_cast<uint32_t*>(w + l.indexA);
+    uint32_t* indexB = reinterpret_cast<uint32_t*>(w + l.indexB);
+    uint8_t* head = w + l.head;
+    long long* pieceBegin = reinterpret_cast<long long*>(w + l.pieceBegin);
+    long long* runBegin = reinterpret_cast<long long*>(w + l.runBegin);
+    dcsg_inspect_component* partial = reinterpret_cast<dcsg_inspect_component*>(w + l.partial);
+    uint64_t* runs = reinterpret_cast<uint64_t*>(w + l.runs);
+    long long* counts = reinterpret_cast<long long*>(w + l.counts);        // {pieces, shell runs}
+    void* temp = w + l.temp;
+    size_t tempBytes;
+    const long long hi = (long long)nh, ti = (long long)nt, vi = (long long)nv;
+    const int vertexBits = bits_for(nv);
+    cudaError_t e;
+    k_inspect_init<<<blocks_for(nv, kThreads), kThreads, 0, s>>>(nv, parent, ref);
+    k_inspect_triangles<<<blocks_for(nt, kThreads), kThreads, 0, s>>>(p.triangles, nt, keysA, fwdA, ref, parent);
+    k_inspect_flatten<<<blocks_for(nv, kThreads), kThreads, 0, s>>>(nv, parent);
+    k_inspect_labels<<<blocks_for(nt, kThreads), kThreads, 0, s>>>(p.triangles, nt, parent, labelA, indexA);
+    // edges; the sorted keys' unique copies go to keysA, free after the sort
+    tempBytes = l.tempBytes;
+    if ((e = cub::DeviceRadixSort::SortPairs(temp, tempBytes, keysA, keysB, fwdA, fwdB, hi, 0, 32 + vertexBits, s)) != cudaSuccess) return e;
+    tempBytes = l.tempBytes;
+    if ((e = cub::DeviceReduce::ReduceByKey(temp, tempBytes, keysB, keysA, InspectHalfEdges(fwdB, InspectHalfEdge()), packed, runs, InspectAdd(),
+                                            hi, s)) != cudaSuccess) return e;
+    tempBytes = l.tempBytes;
+    if ((e = cub::DeviceReduce::Reduce(temp, tempBytes, thrust::make_transform_iterator(InspectCount(0), InspectEdgeTerm{keysA, packed, runs}),
+                                       &p.totals->e, hi, InspectEdgeSum(), dcsg_inspect_edge_sums{}, s)) != cudaSuccess) return e;
+    // components: pieces of the sorted sequence, then the shells' runs of pieces (the two counts are read back for the grids)
+    const InspectTriangleTerm term{p.vertices, p.triangles};
+    tempBytes = l.tempBytes;
+    if ((e = cub::DeviceRadixSort::SortPairs(temp, tempBytes, labelA, labelB, indexA, indexB, ti, 0, vertexBits, s)) != cudaSuccess) return e;
+    k_inspect_piece_heads<<<blocks_for(nt, kThreads), kThreads, 0, s>>>(labelB, nt, head);
+    tempBytes = l.tempBytes;
+    if ((e = cub::DeviceSelect::Flagged(temp, tempBytes, InspectCount(0), head, pieceBegin, counts, ti, s)) != cudaSuccess) return e;
+    k_inspect_run_heads<<<blocks_for(nt, kThreads), kThreads, 0, s>>>(labelB, nt, pieceBegin, counts, head);
+    tempBytes = l.tempBytes;
+    if ((e = cub::DeviceSelect::Flagged(temp, tempBytes, InspectCount(0), head, runBegin, counts + 1, ti, s)) != cudaSuccess) return e;
+    long long h[2];
+    if ((e = cudaMemcpyAsync(h, counts, sizeof(h), cudaMemcpyDeviceToHost, s)) != cudaSuccess) return e;
+    if ((e = cudaStreamSynchronize(s)) != cudaSuccess) return e;
+    if (h[0] > 0x7fffffffll) return cudaErrorInvalidValue;         // cub's segment counts are int
+    tempBytes = l.tempBytes;
+    if ((e = cub::DeviceSegmentedReduce::Reduce(temp, tempBytes, InspectComponentTerms(indexB, InspectComponentTerm{term}), partial, (int)h[0],
+                                                pieceBegin, InspectEnds(InspectCount(0), InspectSegmentEnd{pieceBegin, counts, ti}),
+                                                InspectComponentSum(), dcsg_inspect_component{}, s)) != cudaSuccess) return e;
+    tempBytes = l.tempBytes;
+    if ((e = cub::DeviceSegmentedReduce::Reduce(temp, tempBytes, (const dcsg_inspect_component*)partial, p.components, (int)h[1], runBegin,
+                                                InspectEnds(InspectCount(0), InspectSegmentEnd{runBegin, counts + 1, h[0]}),
+                                                InspectComponentSum(), dcsg_inspect_component{}, s)) != cudaSuccess) return e;
+    if ((e = cudaMemcpyAsync(&p.totals->componentRuns, counts + 1, 8, cudaMemcpyDeviceToDevice, s)) != cudaSuccess) return e;
+    // sums
+    dcsg_inspect_vertex_sums v0 = {};
+    for (int c = 0; c < 3; ++c) { v0.lo[c] = INFINITY; v0.hi[c] = -INFINITY; }
+    tempBytes = l.tempBytes;
+    if ((e = cub::DeviceReduce::Reduce(temp, tempBytes, thrust::make_transform_iterator(InspectCount(0), InspectVertexTerm{p.vertices, ref, parent}),
+                                       &p.totals->v, vi, InspectVertexSum(), v0, s)) != cudaSuccess) return e;
+    tempBytes = l.tempBytes;
+    if ((e = cub::DeviceReduce::Reduce(temp, tempBytes, thrust::make_transform_iterator(InspectCount(0), term), &p.totals->t, ti,
+                                       InspectTriangleSum(), dcsg_inspect_triangle_sums{}, s)) != cudaSuccess) return e;
     return cudaGetLastError();
 }

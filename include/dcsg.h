@@ -278,6 +278,42 @@ int  dcsg_mesh_orient(dcsg_ctx* ctx, dcsg_mesh* mesh);
 #define DCSG_EXPORT_OUTWARD 1
 int  dcsg_set_export_flags(dcsg_ctx* ctx, int flags);
 
+/* ---- mesh inspection (no reference counterpart: the reference never checks the mesh it writes; DESIGN.md 7d) -------------------
+ * dcsg_mesh_inspect reports whether a mesh is a closed, consistently wound solid, and its area, volume, centre of mass and
+ * extents, computed on the device from d_vertices, d_triangles and the two counts alone.  It works on every mesh the library
+ * hands out: uniform or adaptive, welded or not, oriented or not, the `local` slab of a sharded extraction (a mesh of its own:
+ * its cut shows as boundary edges) and the borrowed `whole` of a gather.  Synchronous; the mesh, its host copies and the
+ * device are left unchanged.  Deterministic: the same bits on every run.  V = num_vertices (< 2^32), T = num_triangles.
+ *   degenerate triangle   two of its three ids are equal; counted, then ignored by everything below
+ *   referenced vertex     used by a non-degenerate triangle; unreferenced_vertices = V - referenced
+ *   non-finite            nonfinite_vertices: referenced vertices with a NaN or Inf coordinate; nonfinite_triangles: non-degenerate
+ *                         triangles with such a corner -- they count for edges and components, not for area, volume, centroid, box
+ *   edges                 the half-edges (a,b), (b,c), (c,a) of the non-degenerate triangles, by undirected pair; per edge k
+ *                         half-edges, f of them with a < b: boundary k = 1, manifold k = 2, non-manifold k >= 3, misoriented
+ *                         k = 2 and f != 1 (both faces traverse the edge the same way)
+ *   per triangle          in double from the float corners: u = b - a, w = c - a, n = u x w, area_t = |n| / 2,
+ *                         vol_t = a . (b x c) / 6, centroid_t = vol_t (a + b + c); zero_area_triangles: finite ones with n = 0
+ *   totals                area, signed_volume = sums over the non-degenerate finite triangles; centroid = sum centroid_t /
+ *                         (4 signed_volume), NaN when the volume is 0; bbox_min / bbox_max = exact float extremes over the
+ *                         referenced finite vertices (+Inf / -Inf without any)
+ *   components            shells: vertices connected through the ids of non-degenerate triangles, counted over referenced
+ *                         vertices and numbered in the order of their smallest vertex id
+ * The component arrays (host, NULL allowed with component_capacity = 0) receive the first min(capacity, components) components'
+ * triangle counts, areas and signed volumes; floor(V / 3) bounds `components`.  A triangle id >= V returns DCSG_ERR_INVALID.
+ * A mesh without triangles gives a zeroed report (NaN centroid, +Inf / -Inf box). */
+typedef struct dcsg_mesh_report {
+    uint64_t num_vertices, num_triangles;
+    uint64_t unreferenced_vertices, nonfinite_vertices;
+    uint64_t degenerate_triangles, zero_area_triangles, nonfinite_triangles;
+    uint64_t edges, boundary_edges, manifold_edges, nonmanifold_edges, misoriented_edges;
+    uint64_t components;
+    double   area, signed_volume, centroid[3];
+    float    bbox_min[3], bbox_max[3];
+} dcsg_mesh_report;
+
+int  dcsg_mesh_inspect(dcsg_ctx* ctx, const dcsg_mesh* mesh, dcsg_mesh_report* report, uint64_t component_capacity,
+                       uint64_t* component_triangles, double* component_area, double* component_signed_volume);
+
 typedef struct dcsg_export_report {
     float    box[6];
     uint64_t num_vertices, num_triangles, num_cells;
