@@ -10,6 +10,7 @@
     python -m designcsg_b200 inspect SCENE_DIR|DESIGN.py [--level L] [--outward] [--components]
                                                                        one JSON line: edge topology, shells, area, volume,
                                                                        centroid and extents of the mesh --ply-indexed writes
+    ... inspect ... --deviation [--subdivision K] [--tolerance T]     ... and the design's SDF sampled over that mesh
     torchrun --nproc-per-node G -m designcsg_b200 export ...          z-slab sharded over G GPUs (dcsg_export_sharded; the
                                                                        same export from a C host: tools/dcsg_mgpu.c)
 """
@@ -143,12 +144,17 @@ def cmd_inspect(args):
     from . import api, build
     if int(os.environ.get("WORLD_SIZE", "1")) > 1:
         raise SystemExit("inspect runs on one GPU: the mesh of a sharded export is never gathered; run it without torchrun")
+    if not 1 <= args.subdivision <= 16:
+        raise SystemExit("--subdivision must be in 1..16, not %d" % args.subdivision)
+    if args.tolerance is not None and not args.tolerance >= 0.0:
+        raise SystemExit("--tolerance must be a number >= 0, not %r" % args.tolerance)
     build.build()
     scene = _scene_dir(args.scene)
     _, search, steps, lo, hi, level, threshold = _export_levels(scene, args.level)
     ctx = api.Context(int(os.environ.get("LOCAL_RANK", "0")))
     ctx.build(scene)
-    mesh = ctx.extract(ctx.bbox(search), level, copy_to_host=False, min_level=lo, max_level=hi, complex_threshold=threshold,
+    box = ctx.bbox(search)
+    mesh = ctx.extract(box, level, copy_to_host=False, min_level=lo, max_level=hi, complex_threshold=threshold,
                        retopologize=True, defer_projection=True)
     if args.outward:
         mesh.orient()
@@ -160,6 +166,12 @@ def cmd_inspect(args):
         if name in report:
             report[name] = report[name].tolist()
     report.update(scene=scene, octree_levels=[lo, hi, level], gd_steps=steps, outward=bool(args.outward))
+    if args.deviation:
+        cell = float(max(box[3:6])) / (1 << level)          # the finest lattice cell
+        tolerance = cell / 10 if args.tolerance is None else args.tolerance
+        dev = mesh.deviation(args.subdivision, tolerance)
+        dev.update(subdivision=args.subdivision, tolerance=tolerance, cell=cell)
+        report["deviation"] = dev
     mesh.free()
     ctx.close()
     print(json.dumps(report))
@@ -190,6 +202,11 @@ def main():
     i.add_argument("--level", type=int, default=0, help="uniform lattice of 2^L cells per side (default: exportConfig.txt's levels)")
     i.add_argument("--outward", action="store_true", help="orient the mesh first, as export --outward does")
     i.add_argument("--components", action="store_true", help="add per-shell triangle counts, areas and signed volumes")
+    i.add_argument("--deviation", action="store_true", help="add the design's SDF sampled over every triangle (dcsg_mesh_deviation)")
+    i.add_argument("--subdivision", type=int, default=4, help="--deviation: samples at (i, j) / K over each triangle, K in 1..16 "
+                   "(default 4)")
+    i.add_argument("--tolerance", type=float, default=None, help="--deviation: |SDF| above which a triangle counts as over "
+                   "tolerance (default: a tenth of the finest lattice cell)")
     i.set_defaults(fn=cmd_inspect)
     args = ap.parse_args()
     args.fn(args)

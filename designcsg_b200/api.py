@@ -70,6 +70,14 @@ class MeshReport(ctypes.Structure):
                 ("bbox_min", ctypes.c_float * 3), ("bbox_max", ctypes.c_float * 3)]
 
 
+class DeviationReport(ctypes.Structure):
+    _fields_ = [(name, ctypes.c_uint64) for name in (
+                    "num_vertices", "num_triangles", "measured_vertices", "measured_triangles", "samples", "nan_samples",
+                    "over_tolerance", "worst_triangle")] + \
+               [(name, ctypes.c_float) for name in ("vertex_max_abs", "min_sdf", "max_sdf", "max_abs")] + \
+               [("worst_point", ctypes.c_float * 3), ("vertex_rms", ctypes.c_double), ("mean_abs", ctypes.c_double)]
+
+
 PROGRESS_STATES = ("IDLE", "ESTIMATING_BOUNDING_BOX", "PERFORMING_CMS", "RETOPOLOGIZING", "GRADIENT_DESCENT", "WRITING_STL",
                    "WRITING_PLY", "COMPLETE")                   # dcsg.h DCSG_PROGRESS_*, reference DesignCSG.cpp:603-614
 PROGRESS_FN = ctypes.CFUNCTYPE(None, ctypes.c_void_p, ctypes.c_int, ctypes.c_uint64, ctypes.c_uint64)
@@ -154,6 +162,7 @@ def load_library():
     lib.dcsg_set_export_flags.argtypes = [vp, ci]
     lib.dcsg_mesh_inspect.argtypes = [vp, ctypes.POINTER(MeshStruct), ctypes.POINTER(MeshReport), ctypes.c_uint64, _u64p,
                                       ctypes.POINTER(ctypes.c_double), ctypes.POINTER(ctypes.c_double)]
+    lib.dcsg_mesh_deviation.argtypes = [vp, ctypes.POINTER(MeshStruct), ci, ctypes.c_float, ctypes.POINTER(DeviationReport), _f32p]
     _lib = lib
     return lib
 
@@ -341,6 +350,24 @@ class Mesh:
         if components:
             n = out["components"]
             out.update(component_triangles=tris[:n], component_area=area[:n], component_signed_volume=vol[:n])
+        return out
+
+    def deviation(self, subdivision=4, tolerance=0.0, per_triangle=False):
+        """dcsg_mesh_deviation: the scene's SDF sampled at the vertices and at (k+1)(k+2)/2 - 3 points inside or on the edges of
+        every triangle (k = subdivision, 1..16), as a dict -- measured vertices / triangles, samples, NaN samples, triangles over
+        `tolerance`, vertex_max_abs / vertex_rms, min_sdf / max_sdf / max_abs, the worst triangle and point, the area-weighted
+        mean_abs.  SDF values, not Euclidean distances.  per_triangle=True adds `triangle_max_abs` (float32, one per triangle).
+        Reads the device arrays; changes nothing."""
+        rep = DeviationReport()
+        tmax = np.empty(self.num_triangles, np.float32) if per_triangle else None
+        self._ctx._check(self._ctx.lib.dcsg_mesh_deviation(self._ctx.h, ctypes.byref(self.c), subdivision, ctypes.c_float(tolerance),
+                                                           ctypes.byref(rep), tmax.ctypes.data_as(_f32p) if per_triangle else None))
+        out = {}
+        for name, kind in DeviationReport._fields_:
+            v = getattr(rep, name)
+            out[name] = [float(x) for x in v] if hasattr(v, "__len__") else (int(v) if kind is ctypes.c_uint64 else float(v))
+        if per_triangle:
+            out["triangle_max_abs"] = tmax
         return out
 
     def write_ply_indexed(self, path, normals=False):

@@ -10,6 +10,14 @@ using namespace dcsg_host;
 
 namespace dcsg_host {
 unsigned long long g_launches = 0;      // kernels launched by this library (claimed as gpu_launches by bench.py)
+
+int eval_device_locked(dcsg_ctx* ctx, cudaKernel_t k, const float* d_xyz, size_t n, float* d_out) {
+    if (n == 0) return DCSG_OK;
+    unsigned long long nn = n;
+    void* args[] = {(void*)&d_xyz, (void*)&d_out, &nn};
+    CUDA_TRY(ctx, launch(k, dim3((unsigned)((n + 255) / 256)), dim3(256), args, ctx->stream, ctx->scene.private_words));
+    return DCSG_OK;
+}
 }
 
 extern "C" {
@@ -53,7 +61,7 @@ void dcsg_destroy(dcsg_ctx* ctx) {
     cudaSetDevice(ctx->device);
     cudaStreamSynchronize(ctx->stream);
     for (DevBuf* b : {&ctx->pts, &ctx->vals, &ctx->axes, &ctx->sign, &ctx->leaf, &ctx->cfail, &ctx->coarse, &ctx->levels, &ctx->alive, &ctx->vinfo,
-                      &ctx->tiles, &ctx->small, &ctx->lattice_values, &ctx->fmt, &ctx->adapt_emit, &ctx->adapt_snap, &ctx->search_bits, &ctx->project_cursor, &ctx->lists, &ctx->masks, &ctx->soup, &ctx->project_list, &ctx->weld, &ctx->orient, &ctx->inspect})
+                      &ctx->tiles, &ctx->small, &ctx->lattice_values, &ctx->fmt, &ctx->adapt_emit, &ctx->adapt_snap, &ctx->search_bits, &ctx->project_cursor, &ctx->lists, &ctx->masks, &ctx->soup, &ctx->project_list, &ctx->weld, &ctx->orient, &ctx->inspect, &ctx->deviation})
         b->release();
     ctx->pinned.release();
     ctx->pinned_small.release();
@@ -258,14 +266,6 @@ int dcsg_set_arbitrary_data(dcsg_ctx* ctx, const float* data, size_t items) {
     items = std::min(items, (size_t)DCSG_ARBITRARY_DATA_POINTS);
     CUDA_TRY(ctx, cudaMemcpyAsync(ctx->d_arbitrary, data, items * 4, cudaMemcpyHostToDevice, ctx->stream));
     CUDA_TRY(ctx, cudaStreamSynchronize(ctx->stream));
-    return DCSG_OK;
-}
-
-static int eval_device_locked(dcsg_ctx* ctx, cudaKernel_t k, const float* d_xyz, size_t n, float* d_out) {
-    if (n == 0) return DCSG_OK;
-    unsigned long long nn = n;
-    void* args[] = {(void*)&d_xyz, (void*)&d_out, &nn};
-    CUDA_TRY(ctx, launch(k, dim3((unsigned)((n + 255) / 256)), dim3(256), args, ctx->stream, ctx->scene.private_words));
     return DCSG_OK;
 }
 

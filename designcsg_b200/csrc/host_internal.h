@@ -3,7 +3,7 @@
 // bounding box, slab plan, preview; host_extract.cu: lattice passes and dcsg_extract; host_files.cu: byte-exact
 // files, the projection / format / copy / write pipeline, the one driver behind dcsg_export, dcsg_export_sharded,
 // dcsg_export_indexed and dcsg_export_sharded_indexed; host_indexed.cu: the weld and the indexed PLY's pipeline;
-// host_inspect.cu: the mesh report; host_comm.cu: the communicator and the sharded search and extraction).  Not part of the ABI (include/dcsg.h is).
+// host_inspect.cu: the mesh report; host_deviation.cu: the mesh's deviation from the design; host_comm.cu: the communicator and the sharded search and extraction).  Not part of the ABI (include/dcsg.h is).
 #pragma once
 #include <cuda_runtime.h>
 #include <nvrtc.h>
@@ -198,7 +198,8 @@ struct dcsg_ctx {
            adapt_emit, adapt_snap, search_bits, project_cursor, project_list, lists, masks, soup,
            weld,                    // dcsg_mesh_weld: sort / scan scratch, then the compacted vertices and normals
            orient,                  // dcsg_mesh_orient: per-cell counts, their prefix and the scan's scratch
-           inspect;                 // dcsg_mesh_inspect: sort / reduction scratch, the component runs, the totals
+           inspect,                 // dcsg_mesh_inspect: sort / reduction scratch, the component runs, the totals
+           deviation;               // dcsg_mesh_deviation: vertex values, per-triangle terms, one chunk's points and values
     dcsg_host::HostBuf pinned, pinned_small, pinned_soup;
     // sparse extraction: `leaf` (as leafAlive) and `alive` are all-zero between extractions -- every sparse
     // extraction zeroes the words it wrote (dcsg_launch_cleanup); anything else that writes them clears this flag
@@ -462,6 +463,8 @@ int indexed_pipeline_locked(dcsg_ctx* ctx, dcsg_mesh* mesh, int gd_steps, bool n
 dcsg_ctx* comm_ctx(const dcsg_comm* c);
 
 // host_context.cu
+// dcsg_k_eval_sdf / dcsg_k_eval_normal on n device points, asynchronous on the context's stream (the scene is built)
+int eval_device_locked(dcsg_ctx* ctx, cudaKernel_t k, const float* d_xyz, size_t n, float* d_out);
 int bbox_locked(dcsg_ctx* ctx, float search_diameter, float* box6, int ixBegin, int ixEnd,
                 int (*reduce)(void* user, int* d_minmax, uint32_t* d_hist, cudaStream_t stream), void* reduce_user);
 int plan_slabs_locked(dcsg_ctx* ctx, const float* box6, int grid_level, int world, int granularity, int* bounds);

@@ -191,6 +191,51 @@ size_t dcsg_inspect_scratch_bytes(uint64_t numVertices, uint64_t numTriangles);
 cudaError_t dcsg_launch_inspect_check(const dcsg_inspect_params& p, cudaStream_t s);
 cudaError_t dcsg_launch_inspect(const dcsg_inspect_params& p, cudaStream_t s);
 
+// Mesh deviation (dcsg_mesh_deviation; definitions in include/dcsg.h and DESIGN.md 7e).  Map kernels around the scene's own
+// point kernel (dcsg_k_eval_sdf, launched by the host): vertex marks, sample points per chunk of triangles, one thread per
+// triangle reducing its values to per-triangle terms, then cub reductions of those terms in a fixed order.
+constexpr int kDeviationMaxK = 16;
+constexpr uint64_t kDeviationChunkSamples = 1ull << 24;     // sample points per chunk: 192 MiB of points + 64 MiB of values
+struct dcsg_deviation_totals {
+    uint64_t measuredVertices, nanVertices, vertexValues;   // vertexValues: measured vertices with a non-NaN value
+    uint64_t measuredTriangles, nanSamples, overTolerance;  // nanSamples: NaN values among the S samples of measured triangles
+    uint64_t worstTriangle;                                 // UINT64_MAX without a non-NaN value
+    float vertexMaxAbs, minSdf, maxSdf, maxAbs;
+    float worstPoint[3];
+    double vertexSumSq, sumAreaMean, sumArea;
+};
+struct dcsg_deviation_params {
+    const float* vertices;
+    const uint32_t* triangles;
+    uint64_t numVertices;                       // < 2^32
+    uint64_t numTriangles;                      // > 0
+    int k;                                      // 1..kDeviationMaxK
+    int samples;                                // S = (k+1)(k+2)/2 - 3
+    uint8_t ij[2 * ((kDeviationMaxK + 1) * (kDeviationMaxK + 2) / 2)];   // (i, j) of sample s
+    float tolerance;
+    void* scratch;                              // dcsg_deviation_scratch_bytes(numVertices, numTriangles, samples) bytes
+    dcsg_deviation_totals* totals;              // device
+};
+// triangles per chunk of sample points
+uint64_t dcsg_deviation_chunk(uint64_t numTriangles, int samples);
+size_t dcsg_deviation_scratch_bytes(uint64_t numVertices, uint64_t numTriangles, int samples);
+// where the host evaluates: the vertices' values (numVertices floats), a chunk's points and values (chunk * samples of each)
+float* dcsg_deviation_vertex_values(const dcsg_deviation_params& p);
+float* dcsg_deviation_points(const dcsg_deviation_params& p);
+float* dcsg_deviation_values(const dcsg_deviation_params& p);
+// the device array of triangle_max_abs (numTriangles floats)
+const float* dcsg_deviation_triangle_max_abs(const dcsg_deviation_params& p);
+// the totals dcsg_launch_inspect_check writes its badIds to
+dcsg_inspect_totals* dcsg_deviation_check_totals(const dcsg_deviation_params& p);
+// marks the vertices that non-degenerate triangles reference
+cudaError_t dcsg_launch_deviation_marks(const dcsg_deviation_params& p, cudaStream_t s);
+// the sample points of triangles [first, first + count) (count <= dcsg_deviation_chunk) into dcsg_deviation_points
+cudaError_t dcsg_launch_deviation_points(const dcsg_deviation_params& p, uint64_t first, uint64_t count, cudaStream_t s);
+// the per-triangle terms of the same triangles from the vertex values and the chunk's values
+cudaError_t dcsg_launch_deviation_triangles(const dcsg_deviation_params& p, uint64_t first, uint64_t count, cudaStream_t s);
+// the reductions of the vertex and triangle terms, then the worst point: totals
+cudaError_t dcsg_launch_deviation_totals(const dcsg_deviation_params& p, cudaStream_t s);
+
 // ---- adaptive octree mode (mesher_kernels.cu "adaptive") ----------------------------------------------
 struct dcsg_adapt_emit_params {
     dcsg_grid g;                    // the slab of sample planes the sign bitmap covers (z0 = its first plane)

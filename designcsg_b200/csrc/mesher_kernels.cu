@@ -1320,6 +1320,213 @@ struct InspectLayout {
     }
 };
 
+// ---------------------------------------------------------------------------------------------
+// mesh deviation (dcsg_launch_deviation_*).  The SDF values come from the scene module's dcsg_k_eval_sdf, which the host
+// launches on the vertices and on every chunk's points: this file only makes the points and reduces the values.
+// ---------------------------------------------------------------------------------------------
+
+// sample (i, j) of triangle (a, b, c) at subdivision k, per coordinate in this order of IEEE operations (-fmad=false)
+__device__ __forceinline__ void deviation_point(const float* a, const float* b, const float* c, int i, int j, int k, float* p) {
+    const float w0 = (float)(k - i - j), wi = (float)i, wj = (float)j, kk = (float)k;
+#pragma unroll
+    for (int d = 0; d < 3; ++d) p[d] = ((a[d] * w0 + b[d] * wi) + c[d] * wj) / kk;
+}
+
+__global__ void __launch_bounds__(kThreads) k_deviation_marks(const uint32_t* __restrict__ tris, uint64_t n, uint8_t* __restrict__ ref) {
+    const uint64_t t = (uint64_t)blockIdx.x * kThreads + threadIdx.x;
+    if (t >= n) return;
+    const uint32_t a = tris[t * 3], b = tris[t * 3 + 1], c = tris[t * 3 + 2];
+    if (!inspect_degenerate(a, b, c)) ref[a] = ref[b] = ref[c] = 1;
+}
+
+// one thread per sample point: point q of the chunk is sample q % S of triangle first + q / S
+__global__ void __launch_bounds__(kThreads) k_deviation_points(const dcsg_deviation_params p, uint64_t first, uint64_t count, float* __restrict__ pts) {
+    const uint64_t q = (uint64_t)blockIdx.x * kThreads + threadIdx.x;
+    if (q >= count * (uint64_t)p.samples) return;
+    const uint64_t t = first + q / (uint64_t)p.samples;
+    const int s = (int)(q % (uint64_t)p.samples);
+    const uint32_t* id = p.triangles + t * 3;
+    float x[3];
+    deviation_point(p.vertices + (uint64_t)id[0] * 3, p.vertices + (uint64_t)id[1] * 3, p.vertices + (uint64_t)id[2] * 3, p.ij[2 * s],
+                    p.ij[2 * s + 1], p.k, x);
+    pts[q * 3] = x[0];
+    pts[q * 3 + 1] = x[1];
+    pts[q * 3 + 2] = x[2];
+}
+
+// Per-triangle terms: triangle_max_abs, the largest |f| of the non-NaN values (-Inf without any) and the first slot that has
+// it (0..2 corners, 3 + s sample s), the exact extremes, NaN samples, and area_t * mean_t and area_t -- zero for a triangle
+// with a NaN value.  Not measured: NaN, -Inf, +Inf / -Inf extremes, zeros.
+struct DeviationTerms {
+    float *tmax, *best, *lo, *hi;
+    double *areaMean, *area;
+    uint8_t *nanSamples, *slot, *measured;
+};
+
+__global__ void __launch_bounds__(kThreads) k_deviation_triangles(const dcsg_deviation_params p, uint64_t first, uint64_t count,
+                                                                  const float* __restrict__ vval, const float* __restrict__ vals,
+                                                                  DeviationTerms d) {
+    const uint64_t i = (uint64_t)blockIdx.x * kThreads + threadIdx.x;
+    if (i >= count) return;
+    const uint64_t t = first + i;
+    const dcsg_inspect_triangle_sums s = InspectTriangleTerm{p.vertices, p.triangles}((long long)t);
+    const bool measured = !s.degenerate && !s.nonfinite;
+    float best = -INFINITY, lo = INFINITY, hi = -INFINITY;
+    int slot = 0xff, nans = 0, nanSamples = 0;
+    double sum = 0.0;
+    if (measured) {
+        const float corner[3] = {vval[p.triangles[t * 3]], vval[p.triangles[t * 3 + 1]], vval[p.triangles[t * 3 + 2]]};
+        const float* v = vals + i * (uint64_t)p.samples;
+        for (int n = 0; n < 3 + p.samples; ++n) {
+            const float x = n < 3 ? corner[n] : v[n - 3];
+            if (isnan(x)) {
+                ++nans;
+                nanSamples += n >= 3;
+                continue;
+            }
+            const float ax = fabsf(x);
+            if (ax > best) { best = ax; slot = n; }
+            lo = min_total(lo, x);
+            hi = max_total(hi, x);
+            sum = sum + (double)ax;
+        }
+    }
+    const bool clean = measured && !nans;
+    d.tmax[t] = clean ? best : NAN;
+    d.best[t] = best;
+    d.lo[t] = lo;
+    d.hi[t] = hi;
+    d.areaMean[t] = clean ? s.area * (sum / (double)(3 + p.samples)) : 0.0;
+    d.area[t] = clean ? s.area : 0.0;
+    d.nanSamples[t] = (uint8_t)nanSamples;
+    d.slot[t] = (uint8_t)slot;
+    d.measured[t] = measured;
+}
+
+struct DeviationVertexSums {
+    uint64_t measured, nan, values;
+    float maxAbs;
+    double sumSq;
+};
+struct DeviationVertexTerm {
+    const float* v;
+    const float* vval;
+    const uint8_t* ref;
+    __device__ DeviationVertexSums operator()(long long i) const {
+        const bool m = ref[i] && isfinite(v[i * 3]) && isfinite(v[i * 3 + 1]) && isfinite(v[i * 3 + 2]);
+        const float x = vval[i];
+        const bool use = m && !isnan(x);
+        return DeviationVertexSums{m, m && isnan(x), use, use ? fabsf(x) : -INFINITY, use ? (double)x * (double)x : 0.0};
+    }
+};
+struct DeviationVertexSum {
+    __device__ DeviationVertexSums operator()(const DeviationVertexSums& a, const DeviationVertexSums& b) const {
+        return DeviationVertexSums{a.measured + b.measured, a.nan + b.nan, a.values + b.values, fmaxf(a.maxAbs, b.maxAbs), a.sumSq + b.sumSq};
+    }
+};
+
+struct DeviationTriangleSums {
+    uint64_t measured, nanSamples, over;
+    float lo, hi, best;
+    uint64_t bestTriangle;                      // the smallest t with this best; UINT64_MAX while best = -Inf
+    double areaMean, area;
+};
+struct DeviationTriangleTerm {
+    DeviationTerms d;
+    float tolerance;
+    __device__ DeviationTriangleSums operator()(long long t) const {
+        const bool m = d.measured[t] != 0;
+        const float tmax = d.tmax[t], best = d.best[t];
+        return DeviationTriangleSums{m, d.nanSamples[t], m && !(tmax <= tolerance), d.lo[t], d.hi[t], best,
+                                     best == -INFINITY ? ~0ull : (uint64_t)t, d.areaMean[t], d.area[t]};
+    }
+};
+// every operation is exact or a sum; the argmax is a maximum over (best, -index), a total order: ties go to the lower index
+struct DeviationTriangleSum {
+    __device__ DeviationTriangleSums operator()(const DeviationTriangleSums& a, const DeviationTriangleSums& b) const {
+        const bool takeB = b.best > a.best || (b.best == a.best && b.bestTriangle < a.bestTriangle);
+        return DeviationTriangleSums{a.measured + b.measured, a.nanSamples + b.nanSamples, a.over + b.over, min_total(a.lo, b.lo),
+                                     max_total(a.hi, b.hi), takeB ? b.best : a.best, takeB ? b.bestTriangle : a.bestTriangle,
+                                     a.areaMean + b.areaMean, a.area + b.area};
+    }
+};
+
+__global__ void k_deviation_finish(const dcsg_deviation_params p, const DeviationTerms d, const DeviationVertexSums* __restrict__ vs,
+                                   const DeviationTriangleSums* __restrict__ ts) {
+    dcsg_deviation_totals& o = *p.totals;
+    o.measuredVertices = vs->measured;
+    o.nanVertices = vs->nan;
+    o.vertexValues = vs->values;
+    o.vertexMaxAbs = vs->maxAbs;
+    o.vertexSumSq = vs->sumSq;
+    o.measuredTriangles = ts->measured;
+    o.nanSamples = ts->nanSamples;
+    o.overTolerance = ts->over;
+    o.minSdf = ts->lo;
+    o.maxSdf = ts->hi;
+    o.maxAbs = ts->best;
+    o.worstTriangle = ts->bestTriangle;
+    o.sumAreaMean = ts->areaMean;
+    o.sumArea = ts->area;
+    float x[3] = {NAN, NAN, NAN};
+    const uint64_t t = ts->bestTriangle;
+    if (t != ~0ull) {
+        const uint32_t* id = p.triangles + t * 3;
+        const int slot = d.slot[t];
+        if (slot < 3) {
+            for (int c = 0; c < 3; ++c) x[c] = p.vertices[(uint64_t)id[slot] * 3 + c];
+        } else {
+            deviation_point(p.vertices + (uint64_t)id[0] * 3, p.vertices + (uint64_t)id[1] * 3, p.vertices + (uint64_t)id[2] * 3,
+                            p.ij[2 * (slot - 3)], p.ij[2 * (slot - 3) + 1], p.k, x);
+        }
+    }
+    for (int c = 0; c < 3; ++c) o.worstPoint[c] = x[c];
+}
+
+using DeviationVertexTerms = thrust::transform_iterator<DeviationVertexTerm, InspectCount>;
+using DeviationTriangleTerms = thrust::transform_iterator<DeviationTriangleTerm, InspectCount>;
+
+// Scratch of the deviation: the vertices' referenced marks and values, the per-triangle terms (35 B per triangle), one chunk's
+// points and values, the id check's totals, the two reductions' results, then cub's temporary storage
+struct DeviationLayout {
+    size_t ref, vval, tmax, best, lo, hi, areaMean, area, nanSamples, slot, measured, pts, vals, check, vsum, tsum, temp, tempBytes, total;
+    DeviationLayout(uint64_t nv, uint64_t nt, int samples) {
+        auto align = [](size_t b) { return (b + 255) & ~(size_t)255; };
+        const uint64_t chunk = dcsg_deviation_chunk(nt, samples) * (uint64_t)samples;
+        size_t o = 0;
+        ref = o; o += align(nv);
+        vval = o; o += align(nv * 4);
+        tmax = o; o += align(nt * 4);
+        best = o; o += align(nt * 4);
+        lo = o; o += align(nt * 4);
+        hi = o; o += align(nt * 4);
+        areaMean = o; o += align(nt * 8);
+        area = o; o += align(nt * 8);
+        nanSamples = o; o += align(nt);
+        slot = o; o += align(nt);
+        measured = o; o += align(nt);
+        pts = o; o += align(chunk * 12);
+        vals = o; o += align(chunk * 4);
+        check = o; o += align(sizeof(dcsg_inspect_totals));
+        vsum = o; o += align(sizeof(DeviationVertexSums));
+        tsum = o; o += align(sizeof(DeviationTriangleSums));
+        size_t a = 0, b = 0;
+        cub::DeviceReduce::Reduce(nullptr, a, DeviationVertexTerms(InspectCount(0), DeviationVertexTerm{}), (DeviationVertexSums*)nullptr,
+                                  (long long)nv, DeviationVertexSum(), DeviationVertexSums{});
+        cub::DeviceReduce::Reduce(nullptr, b, DeviationTriangleTerms(InspectCount(0), DeviationTriangleTerm{}), (DeviationTriangleSums*)nullptr,
+                                  (long long)nt, DeviationTriangleSum(), DeviationTriangleSums{});
+        tempBytes = std::max(a, b);
+        temp = o; o += align(tempBytes);
+        total = o;
+    }
+    DeviationTerms terms(void* scratch) const {
+        uint8_t* w = static_cast<uint8_t*>(scratch);
+        return DeviationTerms{reinterpret_cast<float*>(w + tmax), reinterpret_cast<float*>(w + best), reinterpret_cast<float*>(w + lo),
+                              reinterpret_cast<float*>(w + hi), reinterpret_cast<double*>(w + areaMean), reinterpret_cast<double*>(w + area),
+                              w + nanSamples, w + slot, w + measured};
+    }
+};
+
 }  // namespace
 
 // persistent grids: `ctas` CTAs (the host passes a multiple of the SM count), never more than there can be tiles
@@ -1538,4 +1745,73 @@ cudaError_t dcsg_launch_inspect(const dcsg_inspect_params& p, cudaStream_t s) {
     if ((e = cub::DeviceReduce::Reduce(temp, tempBytes, thrust::make_transform_iterator(InspectCount(0), term), &p.totals->t, ti,
                                        InspectTriangleSum(), dcsg_inspect_triangle_sums{}, s)) != cudaSuccess) return e;
     return cudaGetLastError();
+}
+
+uint64_t dcsg_deviation_chunk(uint64_t nt, int samples) {
+    return samples ? std::min<uint64_t>(nt, std::max<uint64_t>(1, kDeviationChunkSamples / (uint64_t)samples)) : nt;
+}
+
+size_t dcsg_deviation_scratch_bytes(uint64_t nv, uint64_t nt, int samples) { return DeviationLayout(nv, nt, samples).total; }
+
+static uint8_t* deviation_at(const dcsg_deviation_params& p, size_t offset) { return static_cast<uint8_t*>(p.scratch) + offset; }
+float* dcsg_deviation_vertex_values(const dcsg_deviation_params& p) {
+    return reinterpret_cast<float*>(deviation_at(p, DeviationLayout(p.numVertices, p.numTriangles, p.samples).vval));
+}
+float* dcsg_deviation_points(const dcsg_deviation_params& p) {
+    return reinterpret_cast<float*>(deviation_at(p, DeviationLayout(p.numVertices, p.numTriangles, p.samples).pts));
+}
+float* dcsg_deviation_values(const dcsg_deviation_params& p) {
+    return reinterpret_cast<float*>(deviation_at(p, DeviationLayout(p.numVertices, p.numTriangles, p.samples).vals));
+}
+const float* dcsg_deviation_triangle_max_abs(const dcsg_deviation_params& p) {
+    return reinterpret_cast<const float*>(deviation_at(p, DeviationLayout(p.numVertices, p.numTriangles, p.samples).tmax));
+}
+
+cudaError_t dcsg_launch_deviation_marks(const dcsg_deviation_params& p, cudaStream_t s) {
+    uint8_t* ref = deviation_at(p, DeviationLayout(p.numVertices, p.numTriangles, p.samples).ref);
+    cudaError_t e = cudaMemsetAsync(ref, 0, p.numVertices, s);
+    if (e != cudaSuccess) return e;
+    k_deviation_marks<<<blocks_for(p.numTriangles, kThreads), kThreads, 0, s>>>(p.triangles, p.numTriangles, ref);
+    return cudaGetLastError();
+}
+
+cudaError_t dcsg_launch_deviation_points(const dcsg_deviation_params& p, uint64_t first, uint64_t count, cudaStream_t s) {
+    if (!count || !p.samples) return cudaSuccess;
+    k_deviation_points<<<blocks_for(count * (uint64_t)p.samples, kThreads), kThreads, 0, s>>>(p, first, count, dcsg_deviation_points(p));
+    return cudaGetLastError();
+}
+
+cudaError_t dcsg_launch_deviation_triangles(const dcsg_deviation_params& p, uint64_t first, uint64_t count, cudaStream_t s) {
+    if (!count) return cudaSuccess;
+    const DeviationLayout l(p.numVertices, p.numTriangles, p.samples);
+    k_deviation_triangles<<<blocks_for(count, kThreads), kThreads, 0, s>>>(p, first, count, reinterpret_cast<const float*>(deviation_at(p, l.vval)),
+                                                                           reinterpret_cast<const float*>(deviation_at(p, l.vals)), l.terms(p.scratch));
+    return cudaGetLastError();
+}
+
+// Two cub reductions in a fixed order (the vertices' terms, the triangles' terms), then one thread writes the totals and the
+// worst point, recomputed from its slot by the points kernel's arithmetic.
+cudaError_t dcsg_launch_deviation_totals(const dcsg_deviation_params& p, cudaStream_t s) {
+    const DeviationLayout l(p.numVertices, p.numTriangles, p.samples);
+    DeviationVertexSums* vs = reinterpret_cast<DeviationVertexSums*>(deviation_at(p, l.vsum));
+    DeviationTriangleSums* ts = reinterpret_cast<DeviationTriangleSums*>(deviation_at(p, l.tsum));
+    const DeviationTerms d = l.terms(p.scratch);
+    size_t tempBytes = l.tempBytes;
+    cudaError_t e;
+    const DeviationVertexSums v0{0, 0, 0, -INFINITY, 0.0};
+    if ((e = cub::DeviceReduce::Reduce(deviation_at(p, l.temp), tempBytes,
+                                       DeviationVertexTerms(InspectCount(0), DeviationVertexTerm{p.vertices, reinterpret_cast<const float*>(deviation_at(p, l.vval)),
+                                                                                                 deviation_at(p, l.ref)}),
+                                       vs, (long long)p.numVertices, DeviationVertexSum(), v0, s)) != cudaSuccess) return e;
+    tempBytes = l.tempBytes;
+    const DeviationTriangleSums t0{0, 0, 0, INFINITY, -INFINITY, -INFINITY, ~0ull, 0.0, 0.0};
+    if ((e = cub::DeviceReduce::Reduce(deviation_at(p, l.temp), tempBytes, DeviationTriangleTerms(InspectCount(0), DeviationTriangleTerm{d, p.tolerance}),
+                                       ts, (long long)p.numTriangles, DeviationTriangleSum(), t0, s)) != cudaSuccess) return e;
+    k_deviation_finish<<<1, 1, 0, s>>>(p, d, vs, ts);
+    return cudaGetLastError();
+}
+
+// the id check of the deviation is the inspection's, on totals of its own in the deviation's scratch
+dcsg_inspect_totals* dcsg_deviation_check_totals(const dcsg_deviation_params& p) {
+    return reinterpret_cast<dcsg_inspect_totals*>(deviation_at(p, DeviationLayout(p.numVertices, p.numTriangles, p.samples).check));
 }

@@ -314,6 +314,51 @@ typedef struct dcsg_mesh_report {
 int  dcsg_mesh_inspect(dcsg_ctx* ctx, const dcsg_mesh* mesh, dcsg_mesh_report* report, uint64_t component_capacity,
                        uint64_t* component_triangles, double* component_area, double* component_signed_volume);
 
+/* ---- mesh deviation (no reference counterpart: DESIGN.md 7e) ------------------------------------------------------------------
+ * dcsg_mesh_deviation samples the scene's SDF f over every triangle of a mesh, on the device: how far the mesh strays from the
+ * design.  f is what dcsg_eval_sdf returns (the checked fast copy, the exact copy as its fallback): every value used here is
+ * bit-identical to dcsg_eval_sdf at the same point.  f is the SDF VALUE, not the Euclidean distance to the surface: the two
+ * agree for exact SDFs (a lone sphere) but not under CSG min / max, smooth minima or non-uniform scale -- hence the names
+ * *_sdf / *_abs.  Reads d_vertices, d_triangles and the two counts, like dcsg_mesh_inspect, and works on the same meshes.
+ * Synchronous; the mesh, its host copies and the device state are left unchanged.  Deterministic: min, max and argmax are
+ * exact, every floating-point sum is a reduction in a fixed order (no atomics).  V = num_vertices (< 2^32), T = num_triangles.
+ *   degenerate triangle   two of its ids are equal (dcsg_mesh_inspect's rule); a triangle id >= V returns DCSG_ERR_INVALID,
+ *                         checked before any vertex is read through it
+ *   measured triangle     not degenerate, and its nine corner floats are finite
+ *   measured vertex       finite, and referenced by a non-degenerate triangle
+ *   samples               k = subdivision, 1 <= k <= 16.  A measured triangle (a, b, c) has its 3 corners, whose values are the
+ *                         vertices' own f(v) (evaluated once per vertex), and S = (k+1)(k+2)/2 - 3 further samples, one per (i, j)
+ *                         with i, j >= 0, i + j <= k other than (0,0), (k,0), (0,k), i ascending then j ascending, at the fp32
+ *                         point p = ((a * (float)(k-i-j) + b * (float)i) + c * (float)j) / (float)k per coordinate, in this
+ *                         order of IEEE operations (no contraction).  A sample on an edge two triangles share is evaluated for
+ *                         each of them.  k = 1: corners only; k = 4: 12 more samples per triangle.
+ *   triangle_max_abs[t]   max |f| over t's 3 + S values; NaN when t is not measured or any of its values is NaN
+ *   report                samples = measured_vertices + S * measured_triangles (the evaluations used), nan_samples = NaN values
+ *                         among them; over_tolerance = measured triangles with triangle_max_abs > tolerance or NaN;
+ *                         vertex_max_abs, vertex_rms = sqrt(sum f^2 / n) over the n non-NaN values of the measured vertices;
+ *                         min_sdf / max_sdf = extremes over the non-NaN values (corners and samples) of the measured triangles,
+ *                         -0 below +0; max_abs = max(max_sdf, -min_sdf); worst_triangle = the smallest t whose non-NaN values
+ *                         reach max_abs (triangle_max_abs[t] == max_abs when t has no NaN value), worst_point = the first of its
+ *                         values in corner-then-(i, j) order that does; mean_abs = sum area_t mean_t / sum area_t over the
+ *                         measured triangles without a NaN value, mean_t = (double sum of |f| over the 3 + S values in sample
+ *                         order) / (3 + S), area_t = dcsg_mesh_inspect's per-triangle area bit for bit; NaN when sum area_t = 0
+ *   empty                 without a measured triangle: the triangle counts 0, min_sdf = +Inf, max_sdf = max_abs = -Inf, worst_triangle =
+ *                         UINT64_MAX, worst_point NaN; without a non-NaN vertex value vertex_max_abs = -Inf, vertex_rms NaN
+ * tolerance >= 0 (a negative or NaN one is DCSG_ERR_INVALID); triangle_max_abs: host array of T floats, or NULL.  Before dcsg_build:
+ * DCSG_ERR_NO_SCENE. */
+typedef struct dcsg_deviation_report {
+    uint64_t num_vertices, num_triangles;
+    uint64_t measured_vertices, measured_triangles;
+    uint64_t samples, nan_samples, over_tolerance;
+    uint64_t worst_triangle;
+    float    vertex_max_abs, min_sdf, max_sdf, max_abs;
+    float    worst_point[3];
+    double   vertex_rms, mean_abs;
+} dcsg_deviation_report;
+
+int  dcsg_mesh_deviation(dcsg_ctx* ctx, const dcsg_mesh* mesh, int subdivision, float tolerance, dcsg_deviation_report* report,
+                         float* triangle_max_abs);
+
 typedef struct dcsg_export_report {
     float    box[6];
     uint64_t num_vertices, num_triangles, num_cells;
