@@ -9,7 +9,7 @@
 using namespace dcsg_host;
 
 namespace dcsg_host {
-unsigned long long g_launches = 0;      // kernels launched by this library (claimed as gpu_launches by bench.py)
+std::atomic<unsigned long long> g_launches{0};      // kernels launched by this library (claimed as gpu_launches by bench.py)
 
 int eval_device_locked(dcsg_ctx* ctx, cudaKernel_t k, const float* d_xyz, size_t n, float* d_out) {
     if (n == 0) return DCSG_OK;
@@ -142,6 +142,9 @@ int dcsg_build(dcsg_ctx* ctx, const char* scene_dir, char* log, size_t log_capac
     std::lock_guard<std::mutex> g(ctx->lock);
     CUDA_TRY(ctx, cudaSetDevice(ctx->device));
     ctx->built = false;
+    // the slab plan follows the last search of THIS scene: a previous scene's surface histogram must not plan the new one's slabs
+    memset(ctx->zhist, 0, sizeof(ctx->zhist));
+    ctx->zhist_c = 0.0f;
     std::string err;
     if (!load_scene(scene_dir, ctx->scene, err)) { copy_log(err, log, log_capacity); return fail(ctx, DCSG_ERR_IO, err); }
     std::vector<char> cubin;

@@ -847,7 +847,6 @@ int dcsg_extract(dcsg_ctx* ctx, const dcsg_extract_cfg* cfg, dcsg_mesh* out) {
     out->d_cell_ids = mp.cellIds;
     out->d_cell_masks = mp.cellMasks;
     out->lattice_samples = evals;
-    st->generation = ++ctx->extract_generation;
     st->uniform = uniform;
     if (!uniform) {
         const uint64_t points = cfg->retopologize ? (1ull << (cfg->grid_level - std::min(cfg->min_level, cfg->max_level))) : 1ull;

@@ -448,7 +448,7 @@ static int view_api(dcsg_ctx* ctx, const dcsg_mesh* mesh, bool ply, const uint8_
 }
 int dcsg_format_stl_view(dcsg_ctx* ctx, const dcsg_mesh* mesh, const uint8_t** bytes, size_t* size) { return view_api(ctx, mesh, false, bytes, size); }
 int dcsg_format_ply_view(dcsg_ctx* ctx, const dcsg_mesh* mesh, const uint8_t** bytes, size_t* size) { return view_api(ctx, mesh, true, bytes, size); }
-unsigned long long dcsg_launch_count(void) { return g_launches; }
+unsigned long long dcsg_launch_count(void) { return g_launches.load(); }
 
 int dcsg_format_stl(dcsg_ctx* ctx, const dcsg_mesh* mesh, uint8_t* out, size_t capacity, size_t* needed) {
     return format_api(ctx, mesh, false, out, capacity, needed);

@@ -11,6 +11,7 @@
 
 #include <algorithm>
 #include <array>
+#include <atomic>
 #include <chrono>
 #include <climits>
 #include <cmath>
@@ -175,7 +176,6 @@ struct dcsg_ctx {
     int export_flags = 0;           // DCSG_EXPORT_*, see dcsg_set_export_flags
 
     bool built = false;
-    uint64_t extract_generation = 0;
     cudaStream_t copy_stream = nullptr;
     cudaStream_t aux_stream = nullptr;      // the clean-up pass of a sparse extraction runs here, under whatever follows on `stream`
     cudaEvent_t aux_ready = nullptr, aux_done = nullptr;
@@ -214,7 +214,7 @@ struct dcsg_ctx {
     void* exchange_user = nullptr;
     bool skip_final_sync = false;   // dcsg_extract returns with its last kernels still queued (stage times are read by the caller)
     uint32_t zhist[512] = {0};      // sign changes of the last bounding-box search per z index: [0,256) in-plane edges, [256,512) z-edges
-    float zhist_c = 0.0f;           // its voxel size
+    float zhist_c = 0.0f;           // its voxel size; 0 = no search of the current scene yet (dcsg_build clears it)
     cudaEvent_t ev[DCSG_STAGE_COUNT + 2] = {nullptr};
 };
 
@@ -236,7 +236,7 @@ inline void report_progress(dcsg_ctx* ctx, int state, uint64_t done, uint64_t to
     if (ctx && ctx->progress) ctx->progress(ctx->progress_user, state, done, total);
 }
 
-extern unsigned long long g_launches;      // kernels launched by this library (claimed as gpu_launches by bench.py)
+extern std::atomic<unsigned long long> g_launches;      // kernels launched by this library (claimed as gpu_launches by bench.py); contexts on several threads count here
 
 // every scene kernel runs 256-thread blocks; smemWords = the design's per-thread private words (Scene::private_words)
 inline cudaError_t launch(cudaKernel_t k, dim3 grid, dim3 block, void** args, cudaStream_t s, int smemWords = 0) {
@@ -412,9 +412,8 @@ private:
 struct MeshStorage {        // owned by a dcsg_mesh through `reserved`
     DevBuf vertices, normals, keys, triangles, cell_ids, cell_masks;
     HostBuf host;
-    // uniform extractions: what dcsg_project_and_format_segments needs to cut the mesh into z-ordered chunks
-    // (valid while the context's tile / vinfo buffers still belong to this extraction)
-    uint64_t generation = 0;
+    // Everything the chunked file pipeline (dcsg_project_and_format_segments) cuts a mesh by is kept here, in the mesh, not in
+    // the context: a mesh can be projected and written after later extractions on its context.
     bool uniform = false;
     // uniform extractions: triangles before each of the slab's own cell layers and vertices before each of its sample planes
     // (own planes, then the halo plane), closed by the totals -- what the chunked file pipeline cuts the mesh by

@@ -439,7 +439,8 @@ int  dcsg_export_sharded_indexed(dcsg_ctx* ctx, dcsg_comm* comm, const char* sce
  * amount of surface, estimated from the per-z sign-change counts of the last dcsg_bbox search on this context.
  * Every rank computes the same plan from its own (identical) search, so nothing is communicated.  bounds has
  * world + 1 entries: rank r meshes layers [bounds[r], bounds[r+1]).  Falls back to equal slabs without an
- * estimate.  No reference counterpart. */
+ * estimate -- before the first search after dcsg_build (a rebuild forgets the previous scene's search).  No reference
+ * counterpart. */
 int  dcsg_plan_slabs(dcsg_ctx* ctx, const float* box6, int grid_level, int world, int granularity, int* bounds);
 
 /* Measurement support (no reference counterpart): achieved non-tensor FP32 rate of this device in TFLOP/s.
